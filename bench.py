@@ -16,7 +16,7 @@ solve), linearisation (dR/du, dR/dm), output J, dJ/du, dJ/dm, one transposed
   --workload p2|hex|motor   the P2 variant, the 3-D cantilever (configs[3]) and the chained motor problem
          (configs[4]) on one GPU (hex also on N), each verified by residual norms + a finite difference
 
-Usage: python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--n 4000]
+Usage: python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--n 4000] [--dump-outputs DIR]
 """
 import argparse
 import json
@@ -260,6 +260,10 @@ class EngineStep:
                          converged=(bool(ni['converged']) or self.kind == 'hex') and li['converged'], J=J)
         return J
 
+    def outputs(self):
+        """What the last step() returned to its caller: the objective, the state and dJ/df."""
+        return dict(J=self.info['J'], u=self.u, dJdf=self.grad)
+
 
 class MotorStep:
     """BASELINE.json configs[4] (examples/em_motor_opt/run_motor_opt.py:94-317) at engine level on the synthetic annulus:
@@ -351,6 +355,40 @@ class MotorStep:
                          converged=bool(ne['converged'] and ni['converged'] and le['converged'] and lm['converged']),
                          fnorm=ne['fnorm'], J=J)
         return J
+
+    def outputs(self):
+        """What the last step() returned to its caller: B-influence, both states and dJ/dg."""
+        return dict(J=self.info['J'], A=self.A, uhat=self.uhat, dJdg=self.grad)
+
+
+DUMP_SAMPLE = 1 << 20          # entries kept of a larger output over all ranks: at most 4 outputs x 8 MB = 32 MB a run
+
+
+def dump_outputs(d, outputs, rank=0, world=1):
+    """--dump-outputs: writes each output of the last timed step as d/<name>.npy (rank r of a multi-GPU run: <name>.rank<r>.npy)
+    in float64.  An output of more than DUMP_SAMPLE // world entries is reduced to that many at sorted indices drawn from a
+    fixed seed, the same indices every run, so that the files of two builds compare entry for entry."""
+    import numpy as np
+    os.makedirs(d, exist_ok=True)
+    keep = DUMP_SAMPLE // world
+    suffix = '' if world == 1 else '.rank%d' % rank
+    for name, a in outputs.items():
+        if hasattr(a, 'cpu'):                                    # device tensor: sample on the device, copy the sample
+            import torch
+            a = a.reshape(-1)
+            if a.numel() > keep:
+                a = a[torch.from_numpy(_sample(a.numel(), keep)).to(a.device)]
+            a = a.cpu().numpy()
+        else:
+            a = np.ravel(a)
+            if a.size > keep:
+                a = a[_sample(a.size, keep)]
+        np.save(os.path.join(d, name + suffix + '.npy'), np.asarray(a, dtype=np.float64))
+
+
+def _sample(n, k):
+    import numpy as np
+    return np.sort(np.random.default_rng(0).choice(n, k, replace=False))
 
 
 def verify(es):
@@ -573,7 +611,13 @@ def main():
                          "configs[1], the 3-D cantilever of configs[3] and the chained motor problem of configs[4], for profiles/")
     ap.add_argument('--precond', default='amg', choices=['amg', 'cheb'], help='motor workload: AMG V-cycle or the round-1 polynomial')
     ap.add_argument('--forcing', type=float, default=0.01, help='motor workload: eta_max of the Eisenstat-Walker inexact Newton (0: every linear solve to rtol)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last one returned as DIR/<name>.npy (float64; an output of more '
+                         'than %d entries / number of ranks as the same seeded sample every run, 32 MB at most in all; rank r of a '
+                         'multi-GPU run writes <name>.rank<r>.npy)' % DUMP_SAMPLE)
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error('--steps must be at least 1')
     if a.workload != 'p1':
         if a.n == N_DEFAULT:
             a.n = dict(p2=2000, hex=256, motor=512)[a.workload]
@@ -603,6 +647,8 @@ def main():
         for _ in range(a.steps):
             _, r = cpu_step(a.n)
         dt = (time.perf_counter() - t0) / a.steps
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs, dict(J=r['J'], u=r['u'], dJdf=r['grad']))
         val = 1.0 / dt
         sample = ('oracle/cpu_path.cpp: C++/OpenMP restatement of the reference path (the reference itself needs dolfinx + '
                   'PETSc/MUMPS, not installable offline) with the GPU arm\'s algorithm (SNES + FMG/GMG-PCG rtol %g) on %d host '
@@ -657,6 +703,8 @@ def main():
     launches = es.launch_count() - l0 - (len(PROBE_MODES) if has_dia else 0)
     counts = [es.p.vcycle_op_probe(m)[1] - c0[m] - 1 for m in PROBE_MODES] if has_dia else None
     clocks = sampler.stop()
+    if a.dump_outputs:
+        dump_outputs(a.dump_outputs, es.outputs(), rank, world)
     kernels = time_kernels(es, counts, a.steps)
     step_info = dict(es.info)
     check = verify(es) if world == 1 else None

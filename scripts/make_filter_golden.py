@@ -1,10 +1,10 @@
 """Golden vectors of the density filter from the REFERENCE ITSELF: imports
-/root/reference/examples/beam_topo_opt/pre_processor/general_filter_model.py (pure numpy / scipy; csdl replaced by femo_b200's
+$FEMO_REFERENCE/examples/beam_topo_opt/pre_processor/general_filter_model.py (pure numpy / scipy; csdl replaced by femo_b200's
 stand-in base classes) and runs its GeneralFilterOperation on a 2-D lattice of cell centres, a 3-D lattice and a scattered
 point set.  Stores the weight matrix (COO triplets in the reference's own order) and the filtered field of a seeded density as
 tests/golden/filter_reference.npz; tests/test_filter_reference.py holds oracle/filter.py to it.
 
-    python scripts/make_filter_golden.py
+    FEMO_REFERENCE=<reference checkout> python scripts/make_filter_golden.py
 """
 import importlib.util
 import os
@@ -15,7 +15,8 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
-REF = '/root/reference/examples/beam_topo_opt/pre_processor/general_filter_model.py'
+REF = (os.path.join(os.path.abspath(os.environ['FEMO_REFERENCE']), 'examples/beam_topo_opt/pre_processor/general_filter_model.py')
+       if os.environ.get('FEMO_REFERENCE') else '')
 
 
 def load_reference_filter(path=REF):
@@ -67,6 +68,8 @@ def run(mod):
 
 
 if __name__ == '__main__':
+    if not REF:
+        sys.exit('set FEMO_REFERENCE to a checkout of the reference femo project')
     path = os.path.join(ROOT, 'tests', 'golden', 'filter_reference.npz')
     np.savez_compressed(path, **run(load_reference_filter()))
     print('->', path)

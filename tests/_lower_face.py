@@ -11,7 +11,8 @@ import types
 
 import numpy as np
 
-REFERENCE = '/root/reference'
+# a checkout of the reference femo project; what runs its code skips without one
+REFERENCE = os.path.abspath(os.environ['FEMO_REFERENCE']) if os.environ.get('FEMO_REFERENCE') else ''
 
 
 class Rec:

@@ -8,7 +8,7 @@ lower-face calls (names, arguments) and every value a callback writes into the C
 Nothing here touches the GPU engine or oracle/: it is about who calls what, in which order, with which arrays, and
 assign-versus-accumulate semantics.  scripts/make_upper_face_trace.py stores the reference's run as
 tests/golden/upper_face_trace.json (the reference cannot travel to the GPU box); tests/test_upper_face.py compares the
-mirrors with it and, where /root/reference exists, regenerates it live.
+mirrors with it and, where $FEMO_REFERENCE names a reference checkout, regenerates it live.
 """
 import importlib
 import importlib.util
@@ -19,7 +19,8 @@ import zlib
 
 import numpy as np
 
-REFERENCE = '/root/reference'
+# a checkout of the reference femo project; what runs its code skips without one
+REFERENCE = os.path.abspath(os.environ['FEMO_REFERENCE']) if os.environ.get('FEMO_REFERENCE') else ''
 
 
 def vec(key, n):

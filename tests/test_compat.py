@@ -13,7 +13,7 @@ def _run(code):
 
 
 def test_reference_import_lines_resolve_to_the_mirrors():
-    """The import lines of /root/reference/examples/*/run_*.py (`from femo.fea.fea_dolfinx import *`,
+    """The import lines of the reference's examples/*/run_*.py (`from femo.fea.fea_dolfinx import *`,
     `from femo.csdl_opt.fea_model import FEAModel`, ...) after `femo_b200.compat.install()`; run in a fresh interpreter
     so that the aliases do not leak into the other tests."""
     out = _run('''
@@ -57,21 +57,23 @@ def test_reference_csdl_layer_defines_over_the_real_lower_face():
     classes) on top of femo_b200.fea through the aliases: FEAModel -> StateModel / OutputModel -> operations are defined for
     the nonlinear Poisson example's registry, with the shapes the engine's spaces report.  (Running the callbacks needs the
     GPU; their call sequence against the lower face is pinned in tests/test_upper_face.py.)"""
-    if not os.path.isdir('/root/reference/femo'):
+    ref = os.path.abspath(os.environ['FEMO_REFERENCE']) if os.environ.get('FEMO_REFERENCE') else ''
+    if not ref or not os.path.isdir(os.path.join(ref, 'femo')):
         import pytest
         pytest.skip('no reference checkout')
     out = _run('''
-import sys, types, importlib.util
+REF = %r
+import os, sys, types, importlib.util
 import femo_b200.compat as c
 c.install(csdl_opt=False)
 from femo_b200.csdl_opt import _csdl_compat as cc
 csdl = types.ModuleType('csdl')
 csdl.Model, csdl.CustomImplicitOperation, csdl.CustomExplicitOperation, csdl.custom = cc.Model, cc.CustomImplicitOperation, cc.CustomExplicitOperation, cc.csdl.custom
 sys.modules['csdl'] = csdl
-pkg = types.ModuleType('femo.csdl_opt'); pkg.__path__ = ['/root/reference/femo/csdl_opt']; sys.modules['femo.csdl_opt'] = pkg
+pkg = types.ModuleType('femo.csdl_opt'); pkg.__path__ = [os.path.join(REF, 'femo', 'csdl_opt')]; sys.modules['femo.csdl_opt'] = pkg
 from femo.csdl_opt.fea_model import FEAModel                 # the reference's file
 import femo.csdl_opt.state_model as sm
-assert sm.__file__.startswith('/root/reference/')
+assert sm.__file__.startswith(os.path.join(REF, ''))
 from femo.fea.fea_dolfinx import *
 from femo_b200.forms.nonlinear_poisson import pdeRes, outputForm
 mesh = createUnitSquareMesh(6)
@@ -87,5 +89,5 @@ assert ops == [('femo.csdl_opt.state_model', 'StateOperation', ['f'], 'u'),
                ('femo.csdl_opt.output_model', 'OutputOperation', ['f', 'u'], 'l2_functional')], ops
 assert sim.vars['f'].shape == (72,) and sim.vars['u'].shape == (49,) and sim.vars['l2_functional'].shape == (1,)
 print('ok')
-''')
+''' % ref)
     assert out.strip().endswith('ok')

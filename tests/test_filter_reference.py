@@ -1,5 +1,5 @@
 """Density filter (SURVEY.md 8f rank 1) held to the reference's own output: tests/golden/filter_reference.npz was produced by
-running /root/reference/examples/beam_topo_opt/pre_processor/general_filter_model.py itself (scripts/make_filter_golden.py).
+running the reference's examples/beam_topo_opt/pre_processor/general_filter_model.py itself (scripts/make_filter_golden.py).
 The oracle's restatement (one KD-tree instead of one per point) must give the same weights and filtered field; the GPU filter
 is compared with the oracle's weights in tests/test_gpu_api.py.  No GPU."""
 import importlib.util
@@ -38,7 +38,7 @@ def test_oracle_filter_equals_the_reference_output(name):
 
 def test_fixture_is_what_the_reference_does_today():
     m = _gen()
-    if not os.path.exists(m.REF):
+    if not m.REF or not os.path.exists(m.REF):
         pytest.skip('no reference checkout')
     live = m.run(m.load_reference_filter())
     z = np.load(GOLD)

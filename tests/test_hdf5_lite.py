@@ -1,9 +1,9 @@
 """femo_b200/fea/hdf5_lite.py: the pure-Python HDF5 reader behind XDMF meshes with HDF5 heavy data (no GPU, no h5py).
 
-Pinned by the one genuine HDF5 file in this image (a MATLAB 7.3 file from scipy's test data, written by the HDF5 library
-itself: user block, superblock 0, symbol-table group, version-1 object header, contiguous float64 data) and by files laid
-out by tests/_hdf5_writer.py for the structures that file does not contain (nested groups, chunked storage with a
-two-level B-tree, edge chunks, shuffle + deflate, integer and big-endian types)."""
+Pinned by a genuine HDF5 file (tests/golden/testhdf5_7.4_GLNX86.mat, a MATLAB 7.3 file copied from SciPy's test data,
+BSD-3-Clause, written by the HDF5 library itself: user block, superblock 0, symbol-table group, version-1 object header,
+contiguous float64 data) and by files laid out by tests/_hdf5_writer.py for the structures that file does not contain
+(nested groups, chunked storage with a two-level B-tree, edge chunks, shuffle + deflate, integer and big-endian types)."""
 import os
 
 import numpy as np
@@ -14,10 +14,7 @@ from _hdf5_writer import write
 
 
 def test_file_written_by_the_hdf5_library():
-    import scipy.io
-    path = os.path.join(os.path.dirname(scipy.io.__file__), 'matlab', 'tests', 'data', 'testhdf5_7.4_GLNX86.mat')
-    if not os.path.exists(path):
-        pytest.skip('scipy test data not installed')
+    path = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'testhdf5_7.4_GLNX86.mat')
     f = hdf5_lite.File(path)
     assert f.base == 512 and f.keys() == ['testdouble']
     a = f['testdouble']

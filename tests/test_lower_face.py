@@ -31,7 +31,7 @@ def _calls(events, name):
 
 
 def test_fixture_is_what_the_reference_does_today(ref):
-    if not os.path.isdir(os.path.join(L.REFERENCE, 'femo')):
+    if not L.REFERENCE or not os.path.isdir(os.path.join(L.REFERENCE, 'femo')):
         pytest.skip('no reference checkout')
     assert json.loads(json.dumps(L.record())) == ref
 
@@ -178,25 +178,52 @@ def test_measures_projection_and_constants(ref):
     assert motor.DOLFIN_EPS == ref['DOLFIN_EPS']
 
 
+LOCATE_GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'locate_dofs_reference.npz')
+
+
+def _locate_inputs():
+    """Seeded vertex cloud of an annulus band and query points near 11 of its vertices (polar and cartesian)."""
+    rng = np.random.default_rng(4)
+    th, r = rng.uniform(0, 2 * np.pi, 40), rng.uniform(0.06, 0.12, 40)
+    nodes = np.stack([r * np.cos(th), r * np.sin(th), np.zeros(40)], axis=1)
+    pick = rng.choice(40, 11, replace=False)
+    polar = np.stack([th[pick], r[pick]], axis=1) + rng.normal(0, 1e-4, (11, 2))
+    cart = nodes[pick, :2] + rng.normal(0, 1e-5, (11, 2))
+    return nodes, pick, polar, cart
+
+
+def test_locate_dofs_equals_the_recorded_reference_output():
+    """locateDOFs / findNodeIndices of the mirror against what the reference's own functions return on the inputs of
+    _locate_inputs(), stored in tests/golden/locate_dofs_reference.npz (held to a live reference run below)."""
+    import types
+    from femo_b200.fea import utils_b200 as ub
+    z = np.load(LOCATE_GOLD)
+    V = types.SimpleNamespace(tabulate_dof_coordinates=lambda: z['nodes'])
+    polar = z['polar'].ravel().copy()
+    assert np.array_equal(ub.locateDOFs(polar, V, input='polar'), z['polar_dofs'])
+    assert np.array_equal(polar, z['polar'].ravel())                        # the mirror leaves its argument alone
+    assert np.array_equal(ub.locateDOFs(z['cart'].copy(), V, input='cartesian'), z['cart_dofs'])
+    assert np.array_equal(ub.findNodeIndices(z['cart'], z['nodes'][:, :2]), z['node_indices'])
+
+
 def test_locate_dofs_equals_the_reference_function():
     """locateDOFs / findNodeIndices (utils_dolfinx.py:126-134,617-641) are plain numpy + KDTree code: the reference's own
-    functions are CALLED here (polar and cartesian input) and the mirror must return the same dof indices.  The reference
+    functions are CALLED here (polar and cartesian input) and must return the stored indices and the mirror's.  The reference
     converts the caller's array to cartesian IN PLACE as a side effect; the mirror leaves its argument alone."""
-    if not os.path.isdir(os.path.join(L.REFERENCE, 'femo')):
+    if not L.REFERENCE or not os.path.isdir(os.path.join(L.REFERENCE, 'femo')):
         pytest.skip('no reference checkout')
     import types
     ref = L.load_reference_utils([])
     from femo_b200.fea import utils_b200 as ub
-    rng = np.random.default_rng(4)
-    th, r = rng.uniform(0, 2 * np.pi, 40), rng.uniform(0.06, 0.12, 40)
-    nodes = np.stack([r * np.cos(th), r * np.sin(th), np.zeros(40)], axis=1)
+    nodes, pick, polar, cart = _locate_inputs()
+    z = np.load(LOCATE_GOLD)
+    assert all(np.array_equal(a, z[k]) for a, k in ((nodes, 'nodes'), (polar, 'polar'), (cart, 'cart')))
     V = types.SimpleNamespace(tabulate_dof_coordinates=lambda: nodes)
-    pick = rng.choice(40, 11, replace=False)
-    polar = np.stack([th[pick], r[pick]], axis=1) + rng.normal(0, 1e-4, (11, 2))
     a0, b0 = polar.ravel().copy(), polar.ravel().copy()
     ia, ib = ref.locateDOFs(a0, V, input='polar'), ub.locateDOFs(b0, V, input='polar')
-    assert np.array_equal(ia, ib) and np.array_equal(ib[0::2] // 2, pick)
+    assert np.array_equal(ia, ib) and np.array_equal(ib[0::2] // 2, pick) and np.array_equal(ia, z['polar_dofs'])
     assert not np.array_equal(a0, polar.ravel()) and np.array_equal(b0, polar.ravel())
-    cart = nodes[pick, :2] + rng.normal(0, 1e-5, (11, 2))
-    assert np.array_equal(ref.locateDOFs(cart.copy(), V, input='cartesian'), ub.locateDOFs(cart.copy(), V, input='cartesian'))
-    assert np.array_equal(ref.findNodeIndices(cart, nodes[:, :2]), ub.findNodeIndices(cart, nodes[:, :2]))
+    ic = ref.locateDOFs(cart.copy(), V, input='cartesian')
+    assert np.array_equal(ic, ub.locateDOFs(cart.copy(), V, input='cartesian')) and np.array_equal(ic, z['cart_dofs'])
+    ni = ref.findNodeIndices(cart, nodes[:, :2])
+    assert np.array_equal(ni, ub.findNodeIndices(cart, nodes[:, :2])) and np.array_equal(ni, z['node_indices'])

@@ -1,9 +1,9 @@
 """The reference's OWN form code, executed: `pdeRes`, `outputForm`, `compliance`, `volume`, `averageFunc` ... are lifted out of
-the example scripts under /root/reference/examples (tests/_ufl_sympy.py: `ast` + a sympy implementation of the UFL operators
+the example scripts under $FEMO_REFERENCE/examples (tests/_ufl_sympy.py: `ast` + a sympy implementation of the UFL operators
 they use) and evaluated cell by cell on the meshes of the exact-integral fixtures.  The global residuals / functionals that come
 out -- and their `sympy.diff` derivatives -- must equal tests/golden/symbolic/*.npz, i.e. the values the oracle (1e-13) and the
 CUDA kernels (1e-12, tests/test_gpu_exact.py) are held to.  This closes the last hand-typed link: the fixtures are what the
-reference's code says, integrated exactly.  Needs the reference checkout (skips on the GPU box); no GPU."""
+reference's code says, integrated exactly.  Needs a reference checkout named by $FEMO_REFERENCE (skips without one); no GPU."""
 import os
 
 import numpy as np
@@ -13,9 +13,22 @@ sp = pytest.importorskip('sympy')
 
 import _ufl_sympy as U   # noqa: E402
 
-REF = '/root/reference/examples'
+REF_ROOT = os.path.abspath(os.environ['FEMO_REFERENCE']) if os.environ.get('FEMO_REFERENCE') else ''
+REF = os.path.join(REF_ROOT, 'examples')
 GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), 'golden', 'symbolic')
-pytestmark = pytest.mark.skipif(not os.path.isdir(REF), reason='no reference checkout')
+needs_reference = pytest.mark.skipif(not REF_ROOT or not os.path.isdir(REF), reason='no reference checkout')
+# the fixture files the tests below were last run against: regenerating a fixture (scripts/make_symbolic_golden.py)
+# fails test_fixtures_are_the_ones_checked_against_the_reference until these tests pass on it and its digest is updated
+CHECKED = {
+    'eb_beam.npz': '57461ae379fd5b731ce75b40d3a3e27f1cced7af7acf1fd2d10244e0adc9fdf7',
+    'motor_em.npz': 'c9ebc38a13e814bea86d07857a352af0b1eaac6c6dda9be7d3d83fdf0244fafd',
+    'motor_mm.npz': 'a54c5d2a880b8c953b6bdd28d5d5b334218e88b70b840fe24c888c2812f3be2f',
+    'nlpoisson_p1.npz': 'fdff29f27d6dc280950910808c6d69f18ef1fc4c3818bf125f3143ae338911d5',
+    'nlpoisson_p2.npz': '5d6c3fb3cf3d8dbffa695fa36fabeee5c45088ba30f2c17336e72b27161eac6a',
+    'poisson_p1.npz': 'be53db5d94ad5916c3ec2c6ddd522b6812842a6f4109e858318118b33101cad6',
+    'simp_hex8.npz': '0f112742358c8f8cf5ba2d0b5f40678e275e3c745fef398d6a59e4c3eb424208',
+    'simp_q1.npz': '37a6b3b078f00e758fef7cb15b01e42505e76b4bdb1070be7fffd1f7bb024ffc',
+}
 TOL = 1e-13
 
 
@@ -25,6 +38,16 @@ def _reset_flags():
     U.NUMERIC = {}
     yield
     U.POLYNOMIAL_COEFFICIENTS = True
+
+
+def test_fixtures_are_the_ones_checked_against_the_reference():
+    """tests/golden/symbolic/*.npz is written by the project's own sympy restatement (tests/test_oracle_symbolic.py); the tests
+    below hold those fixtures to the reference's form code where a checkout is at hand.  Without one, the fixtures must still
+    be the ones those tests passed on."""
+    import hashlib
+    for name, digest in CHECKED.items():
+        with open(os.path.join(GOLD, name), 'rb') as f:
+            assert hashlib.sha256(f.read()).hexdigest() == digest, name
 
 
 def _num(exprs, tab):
@@ -75,6 +98,7 @@ def _tri_cells(z):
     return out, sorted(cnt)
 
 
+@needs_reference
 def test_poisson_forms_as_written_in_the_example():
     """examples/poisson_opt/run_poisson_opt.py: pdeRes(u, v, f) :136 (strong BCs are not part of the form), outputForm(u, f, u_ex) :115."""
     ns = U.load_defs(os.path.join(REF, 'poisson_opt', 'run_poisson_opt.py'))
@@ -96,6 +120,7 @@ def test_poisson_forms_as_written_in_the_example():
 
 
 @pytest.mark.parametrize('degree', [1, 2])
+@needs_reference
 def test_nonlinear_poisson_forms_as_written_in_the_example(degree):
     """examples/nonlinear_poisson_opt/run_nonlinear_poisson_opt.py: pdeRes(u, v, f, u_exact=..., weak_bc=True, sym=True) :196-197,
     outputForm(u, f, u_ex) :172, with the fixture's polynomial u_exact (the example's sin field is not polynomial)."""
@@ -126,6 +151,7 @@ def test_nonlinear_poisson_forms_as_written_in_the_example(degree):
     _compare(z, R, [J], Us, Fs, _table(z, Us, Fs))
 
 
+@needs_reference
 def test_beam_forms_as_written_in_the_example():
     """examples/beam_thickness_opt/run_thickness_opt_cantilever_beam.py: pdeRes(u, v, t, f, ds_(100), E, width) :127-131,
     compliance(u, f, ds_(100)) :135, volume(t, width, L) :137; Hermite-3 with reference-derivative slope dofs."""
@@ -159,6 +185,7 @@ def test_beam_forms_as_written_in_the_example():
 
 
 @pytest.mark.parametrize('name', ['simp_q1', 'simp_hex8'])
+@needs_reference
 def test_simp_forms_as_written_in_the_example(name):
     """examples/beam_topo_opt/run_topo_opt_cantilever_beam.py: pdeRes(u, v, rho, f, dss=ds_(100), method='SIMP') :102-107,
     averageFunc(rho) :111, compliance(u, f, dss=ds_(100)) :113-115.  The form is written for any dimension (`len(u)`,
@@ -209,7 +236,7 @@ def _motor_namespace():
     from a data table at import time)."""
     import json
     fit = json.load(open(os.path.join(os.path.dirname(GOLD), '..', '..', 'femo_b200', 'forms', 'bh_fit.json')))
-    utils = U.load_defs('/root/reference/femo/fea/utils_dolfinx.py')
+    utils = U.load_defs(os.path.join(REF_ROOT, 'femo', 'fea', 'utils_dolfinx.py'))
     perm = U.load_defs(os.path.join(REF, 'em_motor_opt', 'permeability', 'piecewise_permeability.py'),
                        extra=dict(linearA=fit['lin'][0], linearB=fit['lin'][1], cubicA=fit['cubic'][0], cubicB=fit['cubic'][1],
                                   cubicC=fit['cubic'][2], cubicD=fit['cubic'][3], popt_exp=fit['exp'], x1=fit['x1'], x2=fit['x2']))
@@ -267,6 +294,7 @@ def _compare_numeric(z, R, Js, Usym, Msym, tab, tol):
         same(U.jac_numeric([Jf], Msym, tab)[0], z['Jm%d_0' % k], 'dJ%d/dm' % k)
 
 
+@needs_reference
 def test_mesh_motion_forms_as_written_in_the_example():
     """motor_pde.pdeResMM(uhat, v, g=..., nitsche=True, sym=True, overpenalty=False, dS_=dS(1000), ds_=ds(1000)) and
     area_form(uhat, dx, ids) as run_motor_opt.py:176-187 calls them; `X("+")` restrictions are rewritten to restricted(X, "+")."""
@@ -295,6 +323,7 @@ def test_mesh_motion_forms_as_written_in_the_example():
     _compare_numeric(z, R, areas, Us, Gs, tab, 1e-12)
 
 
+@needs_reference
 def test_magnetostatics_forms_as_written_in_the_example():
     """motor_pde.pdeResEM(u, v, uhat, iq, dx, p, s, Hc, vacuum_perm, angle, g=0, nitsche=True, sym=True, overpenalty=False, ds_=ds)
     and B_power_form(u, uhat, n, dx, [1, 2]) as run_motor_opt.py:276-291 calls them -- RelativePermeability, JS, the 216

@@ -32,8 +32,8 @@ def mirror():
 
 
 def test_fixture_is_what_the_reference_does_today(reference):
-    """Where the reference checkout is present (this container, not the GPU box) the committed trace is regenerated from it."""
-    if not os.path.isdir(os.path.join(U.REFERENCE, 'femo')):
+    """Where $FEMO_REFERENCE names a reference checkout the committed trace is regenerated from it."""
+    if not U.REFERENCE or not os.path.isdir(os.path.join(U.REFERENCE, 'femo')):
         pytest.skip('no reference checkout')
     world = U.World()
     live = json.loads(json.dumps(U.scenario(world, U.load_reference(world))))
