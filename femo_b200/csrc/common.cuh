@@ -27,7 +27,7 @@ int set_err(int code, const std::string &msg);
 // Environment switches (debug / test toggles) are looked up once per C-ABI call, not per kernel launch: getenv is a
 // linear scan of the environment and the solver enqueues a few thousand launches per step.
 struct EnvFlags {
-    bool no_bsr = false, no_dia = false, no_overlap = false, no_mgfused = false, no_lattice_asm = false, no_graph = false, force_graph = false;
+    bool no_bsr = false, no_dia = false, no_overlap = false, no_mgfused = false, no_mgsweep = false, no_lattice_asm = false, no_graph = false, force_graph = false;
     long long overlap_min_rows = 1 << 20, mgfused_max_rows = 20000, graph_max_rows = 1 << 20;
     long long mgfused_small_rows = 0;        // fused V-cycle ops up to this many rows run on ONE CTA (FEMO_MGFUSED_SMALL_ROWS); off:
                                              // measured slower (4096: 50.5 ms against 46.9 ms per step, profiles/r02_summary.md)
@@ -266,4 +266,5 @@ struct femo_problem {
     long long graph_replays = 0;             // PCG iterations replayed from a captured CUDA graph
     long long dia_count[4] = {0, 0, 0, 0};   // launches of the DIA operator kernel on this level, by mode
     long long dia64_count[2] = {0, 0};       // launches of the fp64 DIA SpMV on this level: with / without the fused dot
+    long long sweep_count[2] = {0, 0};       // launches of the fused level sweeps (mgsweep.cuh) on this level: down / up
 };

@@ -29,6 +29,7 @@ void refresh_env() {
     g_env.no_bsr = getenv("FEMO_BSR") == nullptr || getenv("FEMO_NO_BSR") != nullptr;
     g_env.no_overlap = getenv("FEMO_NO_OVERLAP") != nullptr;
     g_env.no_mgfused = getenv("FEMO_NO_MGFUSED") != nullptr;
+    g_env.no_mgsweep = getenv("FEMO_NO_MGSWEEP") != nullptr;
     g_env.no_lattice_asm = getenv("FEMO_NO_LATTICE_ASM") != nullptr;
     g_env.no_graph = getenv("FEMO_NO_GRAPH") != nullptr;
     g_env.force_graph = getenv("FEMO_GRAPH") != nullptr;
@@ -918,6 +919,7 @@ static int lattice_jacobian(femo_problem *p, double *d_vals, double *d_vals_bc, 
 #include "stencil.cuh"
 #include "multigrid.cuh"
 #include "mgfused.cuh"
+#include "mgsweep.cuh"
 #include "amg.cuh"
 #include "krylov.cuh"
 #include "gmres.cuh"
@@ -2618,15 +2620,29 @@ int femo_amg_level_values(femo_problem *p, int level, int which, int from_device
 }
 
 /* measurement hook (bench.py roofline): ONE launch of the fine-level V-cycle operator kernel in `mode`
- * (0 residual, 1 first / 2 later Chebyshev step, 3 fused zero-guess pre-smoother) on the hierarchy the last
- * multigrid-preconditioned solve set up; vectors are the solver's own work vectors.  info[0] = algorithmic bytes of the
- * launch, info[1] = fine-level launches of this mode so far (before this one). */
+ * (0 residual, 1 first / 2 later Chebyshev step, 3 fused zero-guess pre-smoother, 6 / 7 down / up level sweep) on the
+ * hierarchy the last multigrid-preconditioned solve set up; vectors are the solver's own work vectors.  info[0] =
+ * algorithmic bytes of the launch, info[1] = fine-level launches of this mode so far (before this one). */
 int femo_vcycle_op_probe(femo_problem *p, int mode, int64_t info[2]) {
     int rc;
     if ((rc = need_device(p))) return rc;
-    if (mode < 0 || mode > 5) return set_err(FEMO_EINVAL, "femo_vcycle_op_probe: mode 0..5");
+    if (mode < 0 || mode > 7) return set_err(FEMO_EINVAL, "femo_vcycle_op_probe: mode 0..7");
     if (!dia_ready(p)) return set_err(FEMO_ESTATE, "femo_vcycle_op_probe: no DIA hierarchy (run a precond=2 solve on a lattice P1 problem first)");
     const int64_t N = p->state.ndofs;
+    if (mode >= 6) {
+        // down: b, dinv, 7 planes read, x_pre written, coarse b written ; up: x_pre, b, 7 planes + dinv read, coarse x read,
+        // x written ; + the Dirichlet marks read once when the level has them
+        const MgParams mp;
+        if (p->mg.empty() || !mgsweep_ok(p, p->mg[0], mp))
+            return set_err(FEMO_ESTATE, "femo_vcycle_op_probe: the fine level does not take the level sweeps");
+        femo_problem *C = p->mg[0];
+        const int64_t nc = C->state.ndofs;
+        int64_t bytes = mode == 6 ? 48 * N + 8 * nc : 56 * N + 8 * nc;
+        if (p->has_bc) bytes += N;
+        if (mode == 6 && C->has_bc) bytes += nc;
+        if (info) { info[0] = bytes; info[1] = p->sweep_count[mode - 6]; }
+        return mode == 6 ? mgsweep_down(p, C, p->kr_r, p->kr_d, mp) : mgsweep_up(p, C, p->kr_r, p->kr_d, p->kr_z, mp);
+    }
     if (mode >= 4) {
         // fp64 planes of the CG recurrence: 7 x 8 B values + x read + y written; mode 4 = fused dot(x, y), 5 = plain
         if (!p->mgl.dia64) return set_err(FEMO_ESTATE, "femo_vcycle_op_probe: no fp64 DIA planes on this problem");

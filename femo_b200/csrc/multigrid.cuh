@@ -248,6 +248,16 @@ struct LatD {
     int nx, nrows, j0;
 };
 
+// value-level expressions of the nested transfers, shared with the fused level sweeps (mgsweep.cuh)
+// xf + P xc at a fine node: a = xc at the coarse node (i>>1, j>>1), a2 = xc at (+oi, +oj); odd = oi | oj
+__device__ __forceinline__ double prolong_nested_val(double xf, double a, double a2, bool odd) {
+    return xf + (odd ? 0.5 * (a + a2) : a);
+}
+// P^T r at a coarse node from the fine residual at the coincident node c and its six stencil neighbours (left to right)
+__device__ __forceinline__ double restrict_nested_val(double c, double l, double r, double d, double u, double dl, double ur) {
+    return c + 0.5 * (l + r + d + u + dl + ur);
+}
+
 // weights of the right-diagonal P1 hat: 1 at coincident nodes, 1/2 along x, y and the (1,1) diagonal
 template <bool CG = false>
 __device__ __forceinline__ void prolong_nested_at(LatD f, LatD c, const double *xc, double *xf, const uint8_t *mask_f, int64_t idx) {
@@ -259,7 +269,8 @@ __device__ __forceinline__ void prolong_nested_at(LatD f, LatD c, const double *
     const int Jl = (gj >> 1) - c.j0;
     if (Jl < 0 || Jl + oj >= c.nrows) return;
     const double a = ldv<CG>(xc + (int64_t)Jl * cw + I);
-    xf[idx] = ldv<CG>(xf + idx) + ((oi | oj) ? 0.5 * (a + ldv<CG>(xc + (int64_t)(Jl + oj) * cw + (I + oi))) : a);
+    const double a2 = (oi | oj) ? ldv<CG>(xc + (int64_t)(Jl + oj) * cw + (I + oi)) : 0.0;
+    xf[idx] = prolong_nested_val(ldv<CG>(xf + idx), a, a2, oi | oj);
 }
 
 __global__ void __launch_bounds__(kThreads)
@@ -285,7 +296,7 @@ __device__ __forceinline__ void restrict_nested_at(LatD f, LatD c, const double 
         const int64_t k = (int64_t)jj * fw + ii;
         return (mask_f && mask_f[k]) ? 0.0 : ldv<CG>(rf + k);
     };
-    rc[idx] = at(i, j) + 0.5 * (at(i - 1, j) + at(i + 1, j) + at(i, j - 1) + at(i, j + 1) + at(i - 1, j - 1) + at(i + 1, j + 1));
+    rc[idx] = restrict_nested_val(at(i, j), at(i - 1, j), at(i + 1, j), at(i, j - 1), at(i, j + 1), at(i - 1, j - 1), at(i + 1, j + 1));
 }
 
 __global__ void __launch_bounds__(kThreads)
@@ -919,8 +930,11 @@ static inline bool nested_pair(const femo_problem *F, const femo_problem *C) {
 static int mg_restrict(femo_problem *L, femo_problem *C, double *rf, double *rc_);
 static int mg_prolong_add(femo_problem *L, femo_problem *C, double *xc, double *xf);
 static int mgfused_vcycle(femo_problem *root, int lv, const double *b, double *x, const MgParams &mp, bool *done);
+static int mgsweep_vcycle(femo_problem *root, int lv, const double *b, double *x, const MgParams &mp, bool *done);
 
-// one V-cycle: level lv solves A x = b approximately from a zero initial guess
+// one V-cycle: level lv solves A x = b approximately from a zero initial guess.  Levels <= FEMO_MGFUSED_MAX_ROWS run
+// as one cooperative kernel (mgfused.cuh); single-GPU DIA levels above that range with a 2:1 nested coarse level run
+// their visit as two stencil sweeps (mgsweep.cuh); every other level takes the per-kernel path below.
 static int mg_vcycle(femo_problem *root, int lv, const double *b, double *x, const MgParams &mp) {
     femo_problem *L = (lv == 0) ? root : root->mg[lv - 1];
     const int nlev = (int)root->mg.size() + 1;
@@ -937,6 +951,11 @@ static int mg_vcycle(femo_problem *root, int lv, const double *b, double *x, con
     {   // coarse levels: the whole sub-V-cycle in one cooperative kernel (mgfused.cuh)
         bool done = false;
         if ((rc = mgfused_vcycle(root, lv, b, x, mp, &done))) return rc;
+        if (done) return FEMO_OK;
+    }
+    {   // large DIA levels: the whole visit in two stencil sweeps around the coarse correction (mgsweep.cuh)
+        bool done = false;
+        if ((rc = mgsweep_vcycle(root, lv, b, x, mp, &done))) return rc;
         if (done) return FEMO_OK;
     }
     femo_problem *C = root->mg[lv];

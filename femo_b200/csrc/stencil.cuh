@@ -10,6 +10,9 @@
 // Row epilogues: the Chebyshev smoother steps of multigrid.cuh are fused into the operator, the
 // Jacobi scaling 1/a_ii is taken from the diagonal plane (no dinv vector), the zero-guess degree-2
 // pre-smoother is ONE kernel, and residual/direction vectors that nobody reads are not written.
+// k_dia_apply serves the V-cycle of multi-GPU slab levels, levels without a 2:1 nested coarse level, the other smoother
+// degrees and the residuals of the full-multigrid start; single-GPU levels above the cooperative coarse kernel's range
+// run the same row arithmetic inside the two level sweeps of mgsweep.cuh.
 //
 // Included by engine.cu after SpmvEpi is defined.
 #pragma once
@@ -89,6 +92,37 @@ struct DiaEpi {
     int a0 = 0, n0 = -1, a1 = 0, n1 = 0;
 };
 
+// Row arithmetic of the V-cycle operator, shared by k_dia_apply and the fused level sweeps (mgsweep.cuh) so that both
+// evaluate the same expression trees (same FMA contraction, same summation order => the same bits).
+// acc = sum_s a_s xv_s as one fma chain, s = 0 .. D-1
+// (a: the fp32 planes, or their exact fp64 conversions)
+template <int D, class P>
+__device__ __forceinline__ double dia_row_acc(const P *a, const double *xv) {
+    double acc = 0.0;
+#pragma unroll
+    for (int s = 0; s < D; ++s) acc = fma((double)a[s], xv[s], acc);
+    return acc;
+}
+// PRE2: xi = dinv_i b_i, acc = sum_s a_s dinv_j b_j ; d0 = c0 xi ; r = b_i - c0 acc ; x = d0 + c1 d0 + c2 dinv_i r
+__device__ __forceinline__ double dia_pre2_row(double c0, double c1, double c2, double xi, double bi, double acc, double di) {
+    const double d0i = c0 * xi;
+    const double r = bi - c0 * acc;
+    return d0i + c1 * d0i + c2 * di * r;
+}
+// PLAIN with a right-hand side: r = b_i - (A x)_i
+__device__ __forceinline__ double dia_resid_row(double bi, double acc) { return bi - acc; }
+// CHEB0: r = b_i - (A x)_i (returned) ; d = c1 dinv_i r
+__device__ __forceinline__ double dia_cheb0_row(double c1, double bi, double acc, double di, double &d) {
+    const double r = bi - acc;
+    d = c1 * di * r;
+    return r;
+}
+// CHEBK: r = rin_i - (A d)_i ; dn = c1 d_i + c2 dinv_i r (returned)
+__device__ __forceinline__ double dia_chebk_row(double c1, double c2, double xi, double rin, double acc, double di, double &r) {
+    r = rin - acc;
+    return c1 * xi + c2 * di * r;
+}
+
 // One thread per row, 32-bit index arithmetic (int32 dofs), and an interior fast path without per-neighbour range
 // checks (only the first and last w+1 rows of a lattice can reach outside [0,n)).  PRE2 gathers the scaled right-hand
 // side c0 * dinv_j * b_j at the 7 neighbours from the dinv plane (no reciprocals, no staging).  PRE2 runs at 0.77 of
@@ -134,26 +168,19 @@ __global__ void __launch_bounds__(kThreads)
             if (MODE == DIA_PRE2) xv[s] *= ok ? (double)__ldg(dinvp + j) : 0.0;
         }
     }
-    double acc = 0.0, xi = 0.0;
-#pragma unroll
-    for (int s = 0; s < D; ++s) {
-        if (s == SD) xi = xv[s];
-        acc = fma((double)a[s], xv[s], acc);
-    }
+    const double acc = dia_row_acc<D>(a, xv), xi = xv[SD];
     if (MODE == DIA_PRE2) {             // xv = dinv_j b_j ; d0 = c0 xv ; r = b_i - A d0 ; x = d0 + c1 d0 + c2 dinv_i r
-        const double d0i = E.c0 * xi;
-        const double r = __ldg(E.b + i) - E.c0 * acc;
-        y[i] = d0i + E.c1 * d0i + E.c2 * di * r;
+        y[i] = dia_pre2_row(E.c0, E.c1, E.c2, xi, __ldg(E.b + i), acc, di);
     } else if (MODE == DIA_PLAIN) {
-        y[i] = E.b ? E.b[i] - acc : acc;
+        y[i] = E.b ? dia_resid_row(E.b[i], acc) : acc;
     } else if (MODE == DIA_CHEB0) {
-        const double r = E.b[i] - acc;
-        E.rout[i] = r;
-        E.dout[i] = E.c1 * di * r;
+        double d;
+        E.rout[i] = dia_cheb0_row(E.c1, E.b[i], acc, di, d);
+        E.dout[i] = d;
     } else {
-        const double r = E.rin[i] - acc;
+        double r;
+        const double dn = dia_chebk_row(E.c1, E.c2, xi, E.rin[i], acc, di, r);
         if (E.rout) E.rout[i] = r;
-        const double dn = E.c1 * xi + E.c2 * di * r;
         if (E.dout) E.dout[i] = dn;
         if (E.xmode == 0) E.xacc[i] += dn;
         else if (E.xmode == 1) E.xacc[i] += xi + dn;

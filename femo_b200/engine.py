@@ -328,7 +328,9 @@ class EngineProblem:
         return out
 
     def vcycle_op_probe(self, mode):
-        """One launch of the fine-level V-cycle operator kernel (bench.py roofline); returns (algorithmic bytes, fine-level launches of this mode so far)."""
+        """One launch of a fine-level V-cycle kernel (bench.py roofline); returns (algorithmic bytes, fine-level launches of
+        this mode so far).  Modes: 0 residual, 1 / 2 Chebyshev steps, 3 fused pre-smoother (fp32 DIA planes), 4 / 5 fp64
+        DIA SpMV with / without the fused dot, 6 / 7 down / up level sweep (smoother, residual and transfer fused)."""
         info = (C.c_int64 * 2)()
         check(lib.femo_vcycle_op_probe(self._h, int(mode), info))
         return int(info[0]), int(info[1])

@@ -320,8 +320,10 @@ int femo_amg_level_values(femo_problem *p, int level, int which, int from_device
 /* Measurement hook for bench.py's roofline (no reference counterpart): ONE launch of a fine-level operator kernel of
  * the last precond=2 solve on the solver's own work vectors.  mode 0 residual, 1 / 2 Chebyshev steps, 3 fused
  * zero-guess pre-smoother (fp32 DIA planes of the V-cycle); 4 / 5 the fp64 DIA SpMV of the CG recurrence with / without
- * the fused dot product.  info[0] receives the algorithmic bytes of that launch (DESIGN.md section 3), info[1] the
- * fine-level launches of that mode so far. */
+ * the fused dot product; 6 / 7 the down / up level sweep of the V-cycle (pre-smoother + residual + restriction /
+ * prolongation + post-smoother in one kernel each; FEMO_ESTATE when the fine level does not take the sweeps).
+ * info[0] receives the algorithmic bytes of that launch (DESIGN.md section 3), info[1] the fine-level launches of that
+ * mode so far. */
 int femo_vcycle_op_probe(femo_problem *p, int mode, int64_t info[2]);
 
 typedef struct femo_newton_opts {
