@@ -200,62 +200,16 @@ static int amg_numeric(femo_problem *p, femo_amg *G, const double *vals) {
     return FEMO_OK;
 }
 
-// Chebyshev-Jacobi smoother of degree deg on [lmax/ratio, lmax] (same recurrence as mg_smooth, multigrid.cuh)
+// Chebyshev-Jacobi smoother of degree deg on [lmax/ratio, lmax], every operator application a CSR-stream SpMV
 static int amg_smooth(femo_problem *p, AmgLevelDev &L, const double *b, double *x, bool zero_guess, int deg, double ratio) {
-    cudaStream_t st = p->stream;
-    const int64_t n = L.n;
-    const int g = red_grid(p, n);
-    const double lmax = L.lmax, lmin = lmax / ratio;
-    const double theta = 0.5 * (lmax + lmin), delta = 0.5 * (lmax - lmin), sigma = theta / delta;
-    double rho = 1.0 / sigma;
-    double *dcur = L.d, *dnext = L.q;
-    const double *rin;
-    int xmode, rc;
-    if (zero_guess) {
-        if (deg <= 1) {
-            k_cheb_first<true><<<g, kThreads, 0, st>>>(b, L.dinv, 1.0 / theta, dcur, x, n);
-            p->launches++;
-            FEMO_CHECK_LAUNCH();
-            return FEMO_OK;
-        }
-        k_cheb_d0<<<g, kThreads, 0, st>>>(b, L.dinv, 1.0 / theta, dcur, n);
-        p->launches++;
-        rin = b;
-        xmode = 2;
-    } else {
-        SpmvEpi E;
-        E.b = b; E.dinv = L.dinv; E.rout = L.r; E.dout = dcur; E.c1 = 1.0 / theta;
-        if ((rc = amg_apply(p, L.rb, L.nrb, L.rowptr, L.col, L.vals, EPI_CHEB0, x, nullptr, E, L.halo))) return rc;
-        if (deg <= 1) {
-            k_axpy<<<g, kThreads, 0, st>>>(1.0, dcur, x, n);
-            p->launches++;
-            FEMO_CHECK_LAUNCH();
-            return FEMO_OK;
-        }
-        rin = L.r;
-        xmode = 1;
-    }
-    for (int k = 2; k <= deg; ++k) {
-        const double rho_new = 1.0 / (2.0 * sigma - rho);
-        SpmvEpi E;
-        E.dinv = L.dinv; E.rin = rin; E.rout = L.r; E.dout = dnext; E.xacc = x;
-        E.c1 = rho_new * rho; E.c2 = 2.0 * rho_new / delta; E.xmode = xmode;
-        if ((rc = amg_apply(p, L.rb, L.nrb, L.rowptr, L.col, L.vals, EPI_CHEBK, dcur, nullptr, E, L.halo))) return rc;
-        std::swap(dcur, dnext);
-        rin = L.r;
-        xmode = 0;
-        rho = rho_new;
-    }
-    return FEMO_OK;
+    return cheb_smooth(p, ChebWork{L.dinv, L.r, L.d, L.q, L.n, L.lmax}, b, x, zero_guess, deg, ratio, false,
+                       [&](int kind, const double *xin, const SpmvEpi &E) {
+                           return amg_apply(p, L.rb, L.nrb, L.rowptr, L.col, L.vals, kind, xin, nullptr, E, L.halo);
+                       });
 }
 
-struct AmgParams {
-    int degree = 2;
-    double ratio = 4.0;
-};
-
 // one V-cycle from a zero initial guess: x ~ A_l^-1 b
-static int amg_vcycle(femo_problem *p, femo_amg *G, int l, const double *b, double *x, const AmgParams &ap) {
+static int amg_vcycle(femo_problem *p, femo_amg *G, int l, const double *b, double *x, const ChebParams &ap) {
     AmgLevelDev &L = G->lv[l];
     cudaStream_t st = p->stream;
     int rc;

@@ -1557,7 +1557,7 @@ static int set_bc_impl(femo_problem *p, const int32_t *dofs, const int32_t *list
 // coarse multigrid levels inherit Dirichlet rows geometrically: a coarse node is
 // constrained when the fine node nearest to it is (homogeneous correction equation)
 static int propagate_bc(femo_problem *root, int start) {
-    const femo_problem *F = (start == 0) ? root : root->mg[start - 1];
+    const femo_problem *F = mg_level(root, start);
     for (size_t lv = (size_t)start; lv < root->mg.size(); ++lv) {
         femo_problem *C = root->mg[lv];
         if (C->replicated && F->slab.active) {
@@ -2674,10 +2674,8 @@ int femo_newton_solve(femo_problem *p, const femo_newton_opts *opts, femo_newton
     double f0 = 0, fn = 0, f_prev = 0, eta_prev = 0;
     bool jac_valid = false;
     // lattice P1 problems solved by GMG-PCG: the Jacobian rows go straight into the DIA planes of the solve
-    DiaMat dtmp;
-    const bool lat_direct = p->lattice_fast && opts->krylov.precond == 2 && opts->krylov.mg_precision == 0 &&
-                            opts->krylov.method == 0 && !p->mg.empty() && p->mgl.vals32 && dia_offsets(p, dtmp) &&
-                            !g_env.no_lattice_asm;
+    const bool lat_direct = opts->krylov.precond == 2 && opts->krylov.mg_precision == 0 && opts->krylov.method == 0 &&
+                            !p->mg.empty() && lattice_dia_direct(p);
     p->mgl.dinv = p->kr_dinv;
     auto eval_F = [&]() -> int {
         int r;

@@ -45,30 +45,11 @@ __global__ void __launch_bounds__(kThreads) k_scale_to(double a, const double *_
     for (int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; k < n; k += (int64_t)gridDim.x * blockDim.x) out[k] = a * in[k];
 }
 
-__global__ void __launch_bounds__(kThreads) k_hadamard(const double *__restrict__ a, const double *__restrict__ b, double *__restrict__ out, int64_t n) {
-    for (int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; k < n; k += (int64_t)gridDim.x * blockDim.x) out[k] = a[k] * b[k];
-}
-
 }  // namespace femo
 
 using namespace femo;
 
 constexpr int kGmresMax = 72;   // S_GM .. S_GM+kGmresMax scalar slots
-
-// Gershgorin bound + inverse diagonal of level 0 for the Chebyshev polynomial preconditioner (precond 1)
-static int cheb_setup(femo_problem *p, const double *vals) {
-    const int64_t n = p->state.ndofs;
-    const DevPattern &D = p->dpat[0];
-    const int g = red_grid(p, n);
-    int rc;
-    p->mgl.vals = const_cast<double *>(vals);
-    k_diag_gershgorin<<<g, kThreads, 0, p->stream>>>(D.rowptr, D.col, vals, p->mgl.dinv, n, p->own_off, p->own_off + p->own_n, p->d_partials);
-    k_max_finalize<<<1, kThreads, 0, p->stream>>>(p->d_partials, g, p->d_scalars, S_TMP2);
-    p->launches += 2;
-    FEMO_CHECK_LAUNCH();
-    if ((rc = allreduce_scalars(p, S_TMP2, 1, true))) return rc;
-    return read_scalars(p, S_TMP2, 1, &p->mgl.lmax);
-}
 
 static int gmres_solve(femo_problem *p, const double *vals, const double *b, double *x, femo_krylov_opts o,
                        femo_krylov_info *info) {
@@ -76,47 +57,16 @@ static int gmres_solve(femo_problem *p, const double *vals, const double *b, dou
     if (!p->gm_basis) return set_err(FEMO_ESTATE, "GMRES basis not reserved for this problem");
     if (o.precond == 2 && p->mg.empty()) o.precond = 0;
     if (o.precond == 3 && !p->d_dense) o.precond = 0;
-    const int pre = o.precond;
+    Precond P = precond_params(o, ChebParams{12, 150.0});
+    P.mg.ratio = MgParams().ratio;       // under GMRES cheb_ratio sets the polynomial and the AMG smoother, not the V-cycle's
     const int m = (o.restart > 1) ? std::min(o.restart, p->gm_restart) : p->gm_restart;
     const int64_t n = p->state.ndofs, o0 = p->own_off, o1 = p->own_off + p->own_n;
     const DevPattern &D = p->dpat[0];
     cudaStream_t st = p->stream;
     const int g = red_grid(p, n);
     double *V = p->gm_basis, *w = p->kr_q, *z = p->kr_z, *r = p->kr_r, *t = p->kr_p;
-    MgParams mp;
-    mp.fp32 = (o.mg_precision == 0);
-    if (o.cheb_degree > 0) mp.degree = o.cheb_degree;
     int rc, spmvs = 0, its = 0;
-    p->mgl.dinv = p->kr_dinv; p->mgl.r = p->kr_w; p->mgl.d = p->kr_d; p->mgl.q = p->wk_extra;
-    const int cdeg = o.cheb_degree > 0 ? o.cheb_degree : 12;
-    const double cratio = o.cheb_ratio > 1.0 ? o.cheb_ratio : 150.0;
-    AmgParams ap;
-    if (o.cheb_degree > 0) ap.degree = o.cheb_degree;
-    if (o.cheb_ratio > 1.0) ap.ratio = o.cheb_ratio;
-    if (pre == 2) {
-        if ((rc = mg_setup(p, vals, mp.fp32))) return rc;
-    } else if (pre == 4) {
-        if ((rc = amg_numeric(p, p->amg, vals))) return rc;
-    } else if (pre == 1) {
-        if ((rc = cheb_setup(p, vals))) return rc;
-    } else if (pre == 3) {
-        k_dense_inverse<<<1, kThreads, 0, st>>>(D.rowptr, D.col, vals, (int)n, p->d_dense_tmp, p->d_dense);
-        p->launches++;
-    } else {
-        k_diag_inv<<<grid_for(n), kThreads, 0, st>>>(D.rowptr, D.col, vals, p->kr_dinv, n);
-        p->launches++;
-    }
-    FEMO_CHECK_LAUNCH();
-    auto precond = [&](const double *in, double *out) -> int {
-        if (pre == 3) k_dense_apply<<<(int)((n * 32 + kThreads - 1) / kThreads), kThreads, 0, st>>>(p->d_dense, in, out, (int)n);
-        else if (pre == 2) return mg_vcycle(p, 0, in, out, mp);
-        else if (pre == 4) return amg_vcycle(p, p->amg, 0, in, out, ap);
-        else if (pre == 1) return mg_smooth(p, in, out, true, cdeg, cratio, false);
-        else k_hadamard<<<g, kThreads, 0, st>>>(p->kr_dinv, in, out, n);
-        p->launches++;
-        FEMO_CHECK_LAUNCH();
-        return FEMO_OK;
-    };
+    if ((rc = precond_setup(p, P, vals, p->wk_extra))) return rc;
     double s2;
     if ((rc = norm2_sq(p, b, &s2))) return rc;
     const double bnorm = std::sqrt(s2), tol = std::max(o.rtol * bnorm, o.atol);
@@ -139,7 +89,7 @@ static int gmres_solve(femo_problem *p, const double *vals, const double *b, dou
         int j = 0;
         for (; j < m && its < o.max_it; ++j) {
             double *vj = V + (int64_t)j * n, *vn = V + (int64_t)(j + 1) * n;
-            if ((rc = precond(vj, z))) return rc;
+            if ((rc = precond_apply(p, P, vj, z))) return rc;
             if ((rc = launch_spmv<false>(p, D.rb, D.nrb, D.rowptr, D.col, vals, z, w, nullptr, nullptr))) return rc;
             ++spmvs;
             for (int pass = 0; pass < 2; ++pass) {          // CGS2
@@ -189,7 +139,7 @@ static int gmres_solve(femo_problem *p, const double *vals, const double *b, dou
         FEMO_CUDA(cudaMemsetAsync(t, 0, sizeof(double) * n, st));
         k_lincomb<<<g, kThreads, 0, st>>>(V, n, j, p->d_scalars, S_GM, 1.0, t, n);
         p->launches++;
-        if ((rc = precond(t, z))) return rc;
+        if ((rc = precond_apply(p, P, t, z))) return rc;
         k_axpy<<<g, kThreads, 0, st>>>(1.0, z, x, n);
         p->launches++;
         FEMO_CHECK_LAUNCH();

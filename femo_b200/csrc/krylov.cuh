@@ -122,11 +122,13 @@ __global__ void k_scalar_op(double *sc, int op) {
     }
 }
 
+__global__ void __launch_bounds__(kThreads) k_hadamard(const double *__restrict__ a, const double *__restrict__ b, double *__restrict__ out, int64_t n) {
+    for (int64_t k = blockIdx.x * (int64_t)blockDim.x + threadIdx.x; k < n; k += (int64_t)gridDim.x * blockDim.x) out[k] = a[k] * b[k];
+}
+
 }  // namespace femo
 
 using namespace femo;
-
-static int cheb_setup(femo_problem *p, const double *vals);
 
 // fine-level rows up to which the PCG iteration is replayed as a CUDA graph (FEMO_GRAPH_MAX_ROWS overrides)
 static int64_t graph_max_rows() { return g_env.graph_max_rows; }
@@ -203,9 +205,87 @@ static int norm2_sq(femo_problem *p, const double *a, double *out) {
     return read_scalars(p, S_TMP0, 1, out);
 }
 
-// Preconditioned CG on the dR/du pattern; `vals` already in the layout to multiply with.
+// Gershgorin bound + inverse diagonal of level 0 for the Chebyshev polynomial preconditioner (precond 1)
+static int cheb_setup(femo_problem *p, const double *vals) {
+    const int64_t n = p->state.ndofs;
+    const DevPattern &D = p->dpat[0];
+    const int g = red_grid(p, n);
+    int rc;
+    p->mgl.vals = const_cast<double *>(vals);
+    k_diag_gershgorin<<<g, kThreads, 0, p->stream>>>(D.rowptr, D.col, vals, p->mgl.dinv, n, p->own_off, p->own_off + p->own_n, p->d_partials);
+    k_max_finalize<<<1, kThreads, 0, p->stream>>>(p->d_partials, g, p->d_scalars, S_TMP2);
+    p->launches += 2;
+    FEMO_CHECK_LAUNCH();
+    if ((rc = allreduce_scalars(p, S_TMP2, 1, true))) return rc;
+    return read_scalars(p, S_TMP2, 1, &p->mgl.lmax);
+}
+
+// Preconditioner of the Krylov drivers (CG and GMRES):
 //   precond 0: Jacobi, 1: Chebyshev polynomial, 2: geometric multigrid V-cycle, 3: explicit dense inverse,
 //   4: smoothed-aggregation AMG V-cycle (amg.cuh)
+struct Precond {
+    int pre = 0;
+    MgParams mg;           // precond 2
+    ChebParams amg;        // precond 4
+    ChebParams poly;       // precond 1: the polynomial on the root, fp64 CSR
+};
+
+// cheb_degree / cheb_ratio of the options override the smoother defaults; `poly`: the solver's own default polynomial
+static Precond precond_params(const femo_krylov_opts &o, ChebParams poly) {
+    Precond P;
+    P.pre = o.precond;
+    P.mg.fp32 = (o.mg_precision == 0);
+    if (o.cheb_degree > 0) P.mg.degree = P.amg.degree = poly.degree = o.cheb_degree;
+    if (o.cheb_ratio > 1.0) P.mg.ratio = P.amg.ratio = poly.ratio = o.cheb_ratio;
+    P.poly = poly;
+    return P;
+}
+
+// set-up for the matrix `vals`.  q: the root's fourth V-cycle work vector (GMRES keeps kr_q for itself);
+// dia_prepared: `vals` was assembled with the fine level's DIA planes (mg_setup's level0_dia)
+static int precond_setup(femo_problem *p, const Precond &P, const double *vals, double *q, bool dia_prepared = false) {
+    const int64_t n = p->state.ndofs;
+    const DevPattern &D = p->dpat[0];
+    cudaStream_t st = p->stream;
+    int rc;
+    p->mgl.dinv = p->kr_dinv;
+    p->mgl.r = p->kr_w;
+    p->mgl.d = p->kr_d;
+    p->mgl.q = q;
+    if (P.pre == 2) {
+        if ((rc = mg_setup(p, vals, P.mg.fp32, dia_prepared))) return rc;
+    } else if (P.pre == 4) {
+        if ((rc = amg_numeric(p, p->amg, vals))) return rc;
+    } else if (P.pre == 1) {
+        if ((rc = cheb_setup(p, vals))) return rc;
+    } else if (P.pre == 3) {
+        k_dense_inverse<<<1, kThreads, 0, st>>>(D.rowptr, D.col, vals, (int)n, p->d_dense_tmp, p->d_dense);
+        p->launches++;
+    } else {
+        k_diag_inv<<<grid_for(n), kThreads, 0, st>>>(D.rowptr, D.col, vals, p->kr_dinv, n);
+        p->launches++;
+    }
+    FEMO_CHECK_LAUNCH();
+    return FEMO_OK;
+}
+
+// out = M^-1 in.  Jacobi is GMRES's: CG folds it into k_cg_init / k_cg_update.
+static int precond_apply(femo_problem *p, const Precond &P, const double *in, double *out) {
+    const int64_t n = p->state.ndofs;
+    cudaStream_t st = p->stream;
+    switch (P.pre) {
+        case 1: return mg_smooth(p, in, out, true, P.poly.degree, P.poly.ratio, false);
+        case 2: return mg_vcycle(p, 0, in, out, P.mg);
+        case 4: return amg_vcycle(p, p->amg, 0, in, out, P.amg);
+        case 3: k_dense_apply<<<(int)((n * 32 + kThreads - 1) / kThreads), kThreads, 0, st>>>(p->d_dense, in, out, (int)n); break;
+        default: k_hadamard<<<red_grid(p, n), kThreads, 0, st>>>(p->kr_dinv, in, out, n); break;
+    }
+    p->launches++;
+    FEMO_CHECK_LAUNCH();
+    return FEMO_OK;
+}
+
+// Preconditioned CG on the dR/du pattern; `vals` already in the layout to multiply with.  Preconditioner: Precond.
 // op_current: the caller guarantees that `vals` is the (BC'd) Jacobian of the coefficients currently bound to the
 // problem (true inside femo_newton_solve, which assembles it itself): hexahedral lattices then apply the operator
 // matrix-free in the recurrence too.  Matrices handed in through femo_linear_solve are always streamed as given.
@@ -214,7 +294,8 @@ static int cg_solve(femo_problem *p, const double *vals, const double *b, double
     default_krylov(o);
     if (o.precond == 2 && p->mg.empty()) o.precond = 0;
     if (o.precond == 3 && !p->d_dense) return set_err(FEMO_ELIMIT, "precond 3 (dense direct) needs N <= 512 on one GPU");
-    const int pre = o.precond;
+    const Precond P = precond_params(o, ChebParams{8, 60.0});
+    const int pre = P.pre;
     const int64_t n = p->state.ndofs, o0 = p->own_off, o1 = p->own_off + p->own_n;
     const DevPattern &D = p->dpat[0];
     // Launch-bound problems replay the PCG iteration from a CUDA graph (below).  The legacy default stream cannot be
@@ -224,55 +305,39 @@ static int cg_solve(femo_problem *p, const double *vals, const double *b, double
     cudaStream_t st = p->stream;
     double *pa = p->d_partials, *pb = p->d_partials + kMaxPartials;
     const int g = red_grid(p, n), go = red_grid(p, p->own_n);
-    MgParams mp;
-    mp.fp32 = (o.mg_precision == 0);
-    if (o.cheb_degree > 0) mp.degree = o.cheb_degree;
-    if (o.cheb_ratio > 1.0) mp.ratio = o.cheb_ratio;
     int rc, np = 0, spmvs = 0;
-    // preconditioner set-up
-    p->mgl.dinv = p->kr_dinv;
-    p->mgl.r = p->kr_w;
-    p->mgl.d = p->kr_d;
-    p->mgl.q = p->kr_q;
-    const int cdeg = o.cheb_degree > 0 ? o.cheb_degree : 8;
-    const double cratio = o.cheb_ratio > 1.0 ? o.cheb_ratio : 60.0;
-    AmgParams ap;
-    if (o.cheb_degree > 0) ap.degree = o.cheb_degree;
-    if (o.cheb_ratio > 1.0) ap.ratio = o.cheb_ratio;
-    if (pre == 2) {
-        if ((rc = mg_setup(p, vals, mp.fp32, dia_prepared))) return rc;
-    } else if (pre == 4) {
-        if ((rc = amg_numeric(p, p->amg, vals))) return rc;
-    } else if (pre == 1) {
-        if ((rc = cheb_setup(p, vals))) return rc;
-    } else if (pre == 3) {
-        k_dense_inverse<<<1, kThreads, 0, st>>>(D.rowptr, D.col, vals, (int)n, p->d_dense_tmp, p->d_dense);
-        p->launches++;
-    } else {
-        k_diag_inv<<<grid_for(n), kThreads, 0, st>>>(D.rowptr, D.col, vals, p->kr_dinv, n);
-        p->launches++;
-    }
-    FEMO_CHECK_LAUNCH();
+    if ((rc = precond_setup(p, P, vals, p->kr_q, dia_prepared))) return rc;
     // ||b||^2
     k_dot<<<go, kThreads, 0, st>>>(b + p->own_off, b + p->own_off, p->own_n, pa);
     p->launches++;
     if ((rc = reduce_to(p, pa, nullptr, go, S_BB, 0))) return rc;
     // multigrid: replace the caller's initial guess by the full-multigrid iterate (discretisation accuracy)
     // full-multigrid start (halves the iteration count here; measured on slabs too: 14 vs 27 iterations per step at N=2)
-    if (pre == 2 && o.restart != 1 && (rc = mg_fmg(p, b, x, mp))) return rc;
-    const bool mf_outer = op_current && pre == 2 && mp.fp32 && hex_matfree_ready(p);
-    const bool dia_outer = pre == 2 && mp.fp32 && p->mgl.dia64_valid && dia_ready(p);     // fp64 planes of `vals` (set-up)
+    if (pre == 2 && o.restart != 1 && (rc = mg_fmg(p, b, x, P.mg))) return rc;
+    const LevelOp vop = level_op(p, P.mg.fp32);
+    const bool mf_outer = op_current && pre == 2 && vop == LevelOp::MATFREE;
+    const bool dia_outer = pre == 2 && p->mgl.dia64_valid && vop == LevelOp::DIA;       // fp64 planes of `vals` (set-up)
     const bool bsr_outer = !mf_outer && !dia_outer && bsr3_ready(p);                     // vector states in 3-D: 3x3 blocks
     if (bsr_outer && (rc = bsr3_convert(p, vals))) return rc;
+    // q = A xin with the recurrence's operator; dot = std::true_type: also the partial sums of xin.q, their count into np
+    auto outer = [&](auto dot, const double *xin, double *q) -> int {
+        constexpr bool DOT = decltype(dot)::value;
+        int *npo = DOT ? &np : nullptr;
+        if (mf_outer) {
+            SpmvEpi E0;
+            const int r = launch_hex_matfree(p, EPI_PLAIN, xin, q, E0);
+            if (r || !DOT) return r;
+            k_dot<<<go, kThreads, 0, st>>>(xin + p->own_off, q + p->own_off, p->own_n, p->d_partials);
+            p->launches++;
+            np = go;
+            return FEMO_OK;
+        }
+        if (dia_outer) return launch_dia64<DOT>(p, xin, q, nullptr, npo);
+        if (bsr_outer) return launch_spmv_bsr3<DOT>(p, xin, q, nullptr, npo);
+        return launch_spmv<DOT>(p, D.rb, D.nrb, D.rowptr, D.col, vals, xin, q, nullptr, npo);
+    };
     // r = b - A x
-    if (mf_outer) {
-        SpmvEpi E0;
-        if ((rc = launch_hex_matfree(p, EPI_PLAIN, x, p->kr_q, E0))) return rc;
-    } else if (dia_outer) {
-        if ((rc = launch_dia64<false>(p, x, p->kr_q, nullptr, nullptr))) return rc;
-    } else if (bsr_outer) {
-        if ((rc = launch_spmv_bsr3<false>(p, x, p->kr_q, nullptr, nullptr))) return rc;
-    } else if ((rc = launch_spmv<false>(p, D.rb, D.nrb, D.rowptr, D.col, vals, x, p->kr_q, nullptr, nullptr))) return rc;
+    if ((rc = outer(std::false_type{}, x, p->kr_q))) return rc;
     ++spmvs;
     if (pre == 0) {
         k_cg_init<<<g, kThreads, 0, st>>>(b, p->kr_q, p->kr_dinv, p->kr_r, p->kr_p, n, o0, o1, pa, pb);
@@ -297,14 +362,7 @@ static int cg_solve(femo_problem *p, const double *vals, const double *b, double
         int r;
         if (pre != 0) {
             // z = M^-1 r ; rz' = r.z ; p = z + beta p
-            if (pre == 3) {
-                k_dense_apply<<<(int)((n * 32 + kThreads - 1) / kThreads), kThreads, 0, st>>>(p->d_dense, p->kr_r, p->kr_z, (int)n);
-                p->launches++;
-            } else if (pre == 1) {
-                if ((r = mg_smooth(p, p->kr_r, p->kr_z, true, cdeg, cratio, false))) return r;
-            } else if (pre == 4) {
-                if ((r = amg_vcycle(p, p->amg, 0, p->kr_r, p->kr_z, ap))) return r;
-            } else if ((r = mg_vcycle(p, 0, p->kr_r, p->kr_z, mp))) return r;
+            if ((r = precond_apply(p, P, p->kr_r, p->kr_z))) return r;
             k_dot<<<go, kThreads, 0, st>>>(p->kr_r + p->own_off, p->kr_z + p->own_off, p->own_n, pa);
             p->launches++;
             if ((r = reduce_to(p, pa, nullptr, go, S_TMP0, 0))) return r;
@@ -316,17 +374,7 @@ static int cg_solve(femo_problem *p, const double *vals, const double *b, double
             p->launches++;
         }
         // q = A p ; alpha = rz / p.q
-        if (mf_outer) {
-            SpmvEpi E0;
-            if ((r = launch_hex_matfree(p, EPI_PLAIN, p->kr_p, p->kr_q, E0))) return r;
-            k_dot<<<go, kThreads, 0, st>>>(p->kr_p + p->own_off, p->kr_q + p->own_off, p->own_n, p->d_partials);
-            p->launches++;
-            np = go;
-        } else if (dia_outer) {
-            if ((r = launch_dia64<true>(p, p->kr_p, p->kr_q, nullptr, &np))) return r;
-        } else if (bsr_outer) {
-            if ((r = launch_spmv_bsr3<true>(p, p->kr_p, p->kr_q, nullptr, &np))) return r;
-        } else if ((r = launch_spmv<true>(p, D.rb, D.nrb, D.rowptr, D.col, vals, p->kr_p, p->kr_q, nullptr, &np))) return r;
+        if ((r = outer(std::true_type{}, p->kr_p, p->kr_q))) return r;
         ++spmvs;
         if ((r = reduce_to(p, p->d_partials, nullptr, np, S_PQ, 0))) return r;
         if ((r = scalar_op(p, 0))) return r;

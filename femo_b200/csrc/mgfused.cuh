@@ -173,8 +173,6 @@ using namespace femo;
 // levels up to this many rows join the cooperative kernel (FEMO_MGFUSED_MAX_ROWS overrides; measured trade-off in DESIGN.md)
 static int64_t mgfused_max_rows() { return g_env.mgfused_max_rows; }
 
-static inline femo_problem *mg_level(femo_problem *root, int lv) { return lv == 0 ? root : root->mg[lv - 1]; }
-
 // (re)build the op list for levels [k0, coarsest] with the smoother parameters of `mp`; called lazily by the first
 // V-cycle after a set-up (the Chebyshev coefficients depend on the level bounds lmax computed there)
 static int mgfused_build(femo_problem *root, const MgParams &mp) {
@@ -190,7 +188,7 @@ static int mgfused_build(femo_problem *root, const MgParams &mp) {
     int k0 = nlev - 1;
     while (k0 > 0) {
         femo_problem *L = mg_level(root, k0 - 1);
-        if (!dia_ready(L) || L->slab.active || L->state.ndofs > mgfused_max_rows() || hex_matfree_ready(L)) break;
+        if (level_op(L, mp.fp32) != LevelOp::DIA || L->slab.active || L->state.ndofs > mgfused_max_rows()) break;
         --k0;
     }
     if (k0 >= nlev - 1) return FEMO_OK;
@@ -199,12 +197,10 @@ static int mgfused_build(femo_problem *root, const MgParams &mp) {
     ops.clear();
     auto bptr = [&](int lv) { return lv == k0 ? (const double *)1 : (const double *)mg_level(root, lv)->mgl.b; };
     auto xptr = [&](int lv) { return lv == k0 ? (double *)2 : mg_level(root, lv)->mgl.x; };
-    struct Coef { double c0, p1, p2, k1, k2; };
-    auto coef = [&](femo_problem *L) {
-        const double lmax = L->mgl.lmax, lmin = lmax / mp.ratio;
-        const double theta = 0.5 * (lmax + lmin), delta = 0.5 * (lmax - lmin), sigma = theta / delta;
-        const double rho = 1.0 / sigma, rho1 = 1.0 / (2.0 * sigma - rho);
-        return Coef{1.0 / theta, rho1 * rho, 2.0 * rho1 / delta, rho1 * rho, 2.0 * rho1 / delta};
+    auto coef = [&](femo_problem *L) {       // degree 2: the PRE2 step and the CHEB0 / CHEBK pair share c0, c1, c2
+        ChebPoly c(L->mgl.lmax, mp.ratio);
+        c.next();
+        return c;
     };
     auto transfer = [&](MgOp &o, femo_problem *F, femo_problem *C) {
         o.nested = nested_pair(F, C) ? 1 : 0;
@@ -214,9 +210,9 @@ static int mgfused_build(femo_problem *root, const MgParams &mp) {
     };
     for (int lv = k0; lv < nlev - 1; ++lv) {        // down sweep
         femo_problem *L = mg_level(root, lv), *C = mg_level(root, lv + 1);
-        const Coef c = coef(L);
+        const ChebPoly c = coef(L);
         MgOp o;
-        o.type = MGO_PRE2; o.A = L->mgl.dia; o.b = bptr(lv); o.y = xptr(lv); o.c0 = c.c0; o.c1 = c.p1; o.c2 = c.p2;
+        o.type = MGO_PRE2; o.A = L->mgl.dia; o.b = bptr(lv); o.y = xptr(lv); o.c0 = c.c0; o.c1 = c.c1; o.c2 = c.c2;
         ops.push_back(o);
         o = MgOp();
         o.type = MGO_RESID; o.A = L->mgl.dia; o.x = xptr(lv); o.b = bptr(lv); o.y = L->mgl.r;
@@ -234,7 +230,7 @@ static int mgfused_build(femo_problem *root, const MgParams &mp) {
     }
     for (int lv = nlev - 2; lv >= k0; --lv) {       // up sweep
         femo_problem *L = mg_level(root, lv), *C = mg_level(root, lv + 1);
-        const Coef c = coef(L);
+        const ChebPoly c = coef(L);
         MgOp o;
         o.type = MGO_PROLONG; o.src = C->mgl.x; o.dst = xptr(lv);
         transfer(o, L, C);
@@ -243,7 +239,7 @@ static int mgfused_build(femo_problem *root, const MgParams &mp) {
         o.type = MGO_CHEB0; o.A = L->mgl.dia; o.x = xptr(lv); o.b = bptr(lv); o.r = L->mgl.r; o.d = L->mgl.d; o.c1 = c.c0;
         ops.push_back(o);
         o = MgOp();
-        o.type = MGO_CHEBK; o.A = L->mgl.dia; o.x = L->mgl.d; o.b = L->mgl.r; o.y = xptr(lv); o.c1 = c.k1; o.c2 = c.k2;
+        o.type = MGO_CHEBK; o.A = L->mgl.dia; o.x = L->mgl.d; o.b = L->mgl.r; o.y = xptr(lv); o.c1 = c.c1; o.c2 = c.c2;
         ops.push_back(o);
     }
     FEMO_CUDA(cudaMemcpyAsync(root->d_mgops, ops.data(), ops.size() * sizeof(MgOp), cudaMemcpyHostToDevice, root->stream));

@@ -263,25 +263,18 @@ using namespace femo;
 // smoother is the fp32 degree-2 Chebyshev polynomial and the level is above the cooperative coarse kernel's range;
 // FEMO_NO_MGSWEEP restores the per-kernel path (A/B switch).
 static bool mgsweep_ok(const femo_problem *L, const femo_problem *C, const MgParams &mp) {
-    return !g_env.no_mgsweep && mp.fp32 && mp.degree == 2 && dia_ready(L) && nested_pair(L, C) && !L->slab.active &&
-           !C->slab.active && !L->gpart.active && !hex_matfree_ready(L) && L->mgl.dia.nd == 7 &&
+    return !g_env.no_mgsweep && mp.degree == 2 && level_op(L, mp.fp32) == LevelOp::DIA && nested_pair(L, C) &&
+           !L->slab.active && !C->slab.active && !L->gpart.active && L->mgl.dia.nd == 7 &&
            L->state.ndofs > g_env.mgfused_max_rows;
 }
 
-// the level's Chebyshev coefficients, computed exactly as mg_smooth computes them
-struct SweepCoef {
-    double c0, c1, c2;
-};
-static SweepCoef mgsweep_coef(const femo_problem *L, const MgParams &mp) {
-    const double lmax = L->mgl.lmax, lmin = lmax / mp.ratio;
-    const double theta = 0.5 * (lmax + lmin), delta = 0.5 * (lmax - lmin), sigma = theta / delta;
-    const double rho = 1.0 / sigma;
-    const double rho1 = 1.0 / (2.0 * sigma - rho);
-    return SweepCoef{1.0 / theta, rho1 * rho, 2.0 * rho1 / delta};
-}
-
-// strips of near-equal even width, and bands of coarse rows sized so that the grid is about one wave of resident CTAs
-static int mgsweep_args(const femo_problem *L, const femo_problem *C, const void *kern, SweepArgs &S, dim3 &grid) {
+// strips of near-equal even width, and bands of coarse rows sized so that the grid is about one wave of resident CTAs;
+// the degree-2 Chebyshev coefficients (both sweeps use c0, c1, c2)
+static int mgsweep_args(const femo_problem *L, const femo_problem *C, const void *kern, const MgParams &mp, SweepArgs &S,
+                        dim3 &grid) {
+    ChebPoly P(L->mgl.lmax, mp.ratio);
+    P.next();
+    S.c0 = P.c0; S.c1 = P.c1; S.c2 = P.c2;
     S.A = L->mgl.dia;
     S.nx = L->mesh.n[0];
     S.ny = L->mesh.n[1];
@@ -303,9 +296,7 @@ static int mgsweep_down(femo_problem *L, femo_problem *C, const double *b, doubl
     SweepArgs S;
     dim3 grid;
     int rc;
-    if ((rc = mgsweep_args(L, C, (const void *)k_mg_down, S, grid))) return rc;
-    const SweepCoef k = mgsweep_coef(L, mp);
-    S.c0 = k.c0; S.c1 = k.c1; S.c2 = k.c2;
+    if ((rc = mgsweep_args(L, C, (const void *)k_mg_down, mp, S, grid))) return rc;
     k_mg_down<<<grid, kSwThreads, 0, L->stream>>>(S, b, xpre, C->mgl.b);
     L->launches++;
     L->sweep_count[0]++;
@@ -318,9 +309,7 @@ static int mgsweep_up(femo_problem *L, femo_problem *C, const double *b, const d
     SweepArgs S;
     dim3 grid;
     int rc;
-    if ((rc = mgsweep_args(L, C, (const void *)k_mg_up, S, grid))) return rc;
-    const SweepCoef k = mgsweep_coef(L, mp);
-    S.c0 = k.c0; S.c1 = k.c1; S.c2 = k.c2;
+    if ((rc = mgsweep_args(L, C, (const void *)k_mg_up, mp, S, grid))) return rc;
     k_mg_up<<<grid, kSwThreads, 0, L->stream>>>(S, b, xpre, C->mgl.x, x);
     L->launches++;
     L->sweep_count[1]++;

@@ -579,6 +579,9 @@ static long long total_launches(const femo_problem *p) {
     return n;
 }
 
+// level lv of the hierarchy: 0 is the root problem itself
+static inline femo_problem *mg_level(femo_problem *root, int lv) { return lv == 0 ? root : root->mg[lv - 1]; }
+
 // d = c * dinv * b   (first Chebyshev direction from a zero initial guess)
 __global__ void __launch_bounds__(kThreads)
     k_cheb_d0(const double *__restrict__ b, const double *__restrict__ dinv, double c, double *__restrict__ d, int64_t n) {
@@ -586,8 +589,6 @@ __global__ void __launch_bounds__(kThreads)
         d[i] = c * dinv[i] * b[i];
 }
 
-// Chebyshev smoother of degree `deg` on level problem L: x ~ A^-1 b.  Every step after the
-// first is ONE kernel: the SpMV A d with the residual/direction/solution updates in its row epilogue.
 // ---- matrix-free SIMP operator on uniform hexahedral lattices ------------------------------------------------
 // y = A x with A = sum_cells rho_c^p K0 (all cells of a level are congruent boxes, so ONE 24x24 unit-modulus element
 // matrix serves the level): no matrix traffic at all, only x, the cell moduli and the Dirichlet marks.  One thread
@@ -712,6 +713,18 @@ __global__ void __launch_bounds__(kThreads) k_to_f32(const double *__restrict__ 
 // ---- DIA (stencil) levels ------------------------------------------------------------------------------------
 static inline bool dia_ready(const femo_problem *L) { return L->mgl.dia_valid; }
 
+// The representation of a level's operator that the V-cycle streams: at fp32 the matrix-free hexahedral operator, else
+// the DIA planes, else the fp32 CSR copy; fp64 CSR otherwise.  Decided per call, not stored: the Chebyshev
+// preconditioner (precond 1) smooths the root at fp64 without a multigrid set-up.  The first two never compete: DIA
+// planes exist on triangle lattices only, the matrix-free operator on hexahedral ones.
+enum class LevelOp { MATFREE, DIA, CSR32, CSR64 };
+static inline LevelOp level_op(const femo_problem *L, bool fp32) {
+    if (fp32 && hex_matfree_ready(L)) return LevelOp::MATFREE;
+    if (fp32 && dia_ready(L)) return LevelOp::DIA;
+    if (fp32 && L->mgl.vals32) return LevelOp::CSR32;
+    return LevelOp::CSR64;
+}
+
 // column offsets of a scalar vertex space on a right-diagonal triangle lattice: the node itself, its x / y
 // neighbours and the two ends of the cell diagonals
 static inline bool dia_offsets(const femo_problem *L, DiaMat &A) {
@@ -725,6 +738,11 @@ static inline bool dia_offsets(const femo_problem *L, DiaMat &A) {
     A.n = L->state.ndofs;
     A.np = (A.n + 31) & ~(int64_t)31;
     return true;
+}
+// the level's Jacobian can be assembled node-centrically straight into its DIA planes (lattice_jacobian with_dia)
+static inline bool lattice_dia_direct(const femo_problem *L) {
+    DiaMat tmp;
+    return L->lattice_fast && L->mgl.vals32 && dia_offsets(L, tmp) && !g_env.no_lattice_asm;
 }
 // floats reserved for the fp32 operator copy of a level: the CSR copy or the DIA planes, whichever is larger
 static inline size_t fp32_copy_len(const femo_problem *L) {
@@ -827,83 +845,136 @@ static int launch_dia64(femo_problem *L, const double *x, double *y, const doubl
     return FEMO_OK;
 }
 
-// the level's SpMV with a fused Chebyshev epilogue, streaming the fp32 copy of the values when requested
-static int mg_spmv_cheb(femo_problem *L, bool fp32, int kind, const double *x, const SpmvEpi &E) {
+// one application of the level operator `op` with the row epilogue `kind`: EPI_PLAIN y = b - A x (b = E.b), or the
+// Chebyshev steps EPI_CHEB0 / EPI_CHEBK, whose outputs E names
+static int level_apply(femo_problem *L, LevelOp op, int kind, const double *x, double *y, const SpmvEpi &E) {
     femo_mg_level &M = L->mgl;
-    if (fp32 && hex_matfree_ready(L)) return launch_hex_matfree(L, kind, x, nullptr, E);
-    if (fp32 && dia_ready(L)) {
-        DiaEpi De;
-        De.b = E.b; De.rin = E.rin; De.rout = E.rout; De.dout = E.dout; De.xacc = E.xacc;
-        De.c1 = E.c1; De.c2 = E.c2; De.xmode = E.xmode;
-        return launch_dia(L, kind == EPI_CHEB0 ? DIA_CHEB0 : DIA_CHEBK, x, nullptr, De);
+    const DevPattern &D = L->dpat[0];
+    switch (op) {
+        case LevelOp::MATFREE: return launch_hex_matfree(L, kind, x, y, E);
+        case LevelOp::DIA: {
+            DiaEpi De;
+            De.b = E.b; De.rin = E.rin; De.rout = E.rout; De.dout = E.dout; De.xacc = E.xacc;
+            De.c1 = E.c1; De.c2 = E.c2; De.xmode = E.xmode;
+            return launch_dia(L, kind == EPI_PLAIN ? DIA_PLAIN : kind == EPI_CHEB0 ? DIA_CHEB0 : DIA_CHEBK, x, y, De);
+        }
+        case LevelOp::CSR32:
+            if (kind == EPI_PLAIN) return launch_spmv<false>(L, D.rb, D.nrb, D.rowptr, D.col, M.vals32, x, y, E.b, nullptr);
+            return launch_spmv_cheb(L, kind, M.vals32, x, E);
+        default:
+            if (kind == EPI_PLAIN) return launch_spmv<false>(L, D.rb, D.nrb, D.rowptr, D.col, M.vals, x, y, E.b, nullptr);
+            return launch_spmv_cheb(L, kind, M.vals, x, E);
     }
-    if (fp32 && M.vals32) return launch_spmv_cheb(L, kind, M.vals32, x, E);
-    return launch_spmv_cheb(L, kind, M.vals, x, E);
 }
 
-static int mg_smooth(femo_problem *L, const double *b, double *x, bool zero_guess, int deg, double ratio, bool fp32) {
-    femo_mg_level &M = L->mgl;
-    const int64_t n = L->state.ndofs;
-    cudaStream_t st = L->stream;
-    const int g = red_grid(L, n);
-    const double lmax = M.lmax, lmin = lmax / ratio;
-    const double theta = 0.5 * (lmax + lmin), delta = 0.5 * (lmax - lmin), sigma = theta / delta;
-    double rho = 1.0 / sigma;
+// degree and interval [lmax / ratio, lmax] of a Chebyshev-Jacobi smoother
+struct ChebParams {
+    int degree = 2;
+    double ratio = 4.0;
+};
+struct MgParams : ChebParams {
+    bool fp32 = true;      // V-cycle SpMVs stream fp32 copies of the level matrices (vectors stay fp64)
+};
+
+// Chebyshev polynomial of the Jacobi-scaled operator on [lmax / ratio, lmax]: d_1 = c0 D^-1 r_0, then every further step
+// d_k = c1 d_{k-1} + c2 D^-1 r_{k-1} with rho_1 = 1 / sigma, rho_k = 1 / (2 sigma - rho_{k-1}).  Every smoother path
+// (cheb_smooth, the fused PRE2 kernel, the level sweeps, the cooperative coarse V-cycle) takes its coefficients from
+// here, so each is the same double.
+struct ChebPoly {
+    double theta, delta, sigma, rho, c0, c1 = 0.0, c2 = 0.0;
+    ChebPoly(double lmax, double ratio) {
+        const double lmin = lmax / ratio;
+        theta = 0.5 * (lmax + lmin);
+        delta = 0.5 * (lmax - lmin);
+        sigma = theta / delta;
+        rho = 1.0 / sigma;
+        c0 = 1.0 / theta;
+    }
+    void next() {          // c1, c2 of the next step
+        const double rho_new = 1.0 / (2.0 * sigma - rho);
+        c1 = rho_new * rho;
+        c2 = 2.0 * rho_new / delta;
+        rho = rho_new;
+    }
+};
+
+// work vectors of a smoothed level (Jacobi scaling, residual, two directions), its rows and its Gershgorin bound
+struct ChebWork {
+    const double *dinv;
+    double *r, *d, *q;
+    int64_t n;
+    double lmax;
+};
+
+// Chebyshev-Jacobi smoother of degree `deg`: x ~ A^-1 b.  Every step after the first is ONE operator application,
+// apply(kind, x, E) with kind EPI_CHEB0 / EPI_CHEBK, that carries the residual / direction / solution updates in its row
+// epilogue.  Kernels run on p's stream and count on p.  drop_last: the last step stores no residual / direction.
+template <class Apply>
+static int cheb_smooth(femo_problem *p, const ChebWork &W, const double *b, double *x, bool zero_guess, int deg, double ratio,
+                       bool drop_last, const Apply &apply) {
+    const int64_t n = W.n;
+    cudaStream_t st = p->stream;
+    const int g = red_grid(p, n);
+    ChebPoly P(W.lmax, ratio);
     int rc;
-    double *dcur = M.d, *dnext = M.q;
+    double *dcur = W.d, *dnext = W.q;
     const double *rin;
     int xmode;
-    const bool dia = fp32 && dia_ready(L) && !hex_matfree_ready(L);
-    if (zero_guess && deg == 2 && dia) {     // d0, the operator and both updates in one kernel
-        const double rho1 = 1.0 / (2.0 * sigma - rho);
-        DiaEpi E;
-        E.b = b; E.c0 = 1.0 / theta; E.c1 = rho1 * rho; E.c2 = 2.0 * rho1 / delta;
-        return launch_dia(L, DIA_PRE2, nullptr, x, E);
-    }
     if (zero_guess) {
         if (deg <= 1) {
-            k_cheb_first<true><<<g, kThreads, 0, st>>>(b, M.dinv, 1.0 / theta, dcur, x, n);
-            L->launches++;
+            k_cheb_first<true><<<g, kThreads, 0, st>>>(b, W.dinv, P.c0, dcur, x, n);
+            p->launches++;
             FEMO_CHECK_LAUNCH();
             return FEMO_OK;
         }
-        k_cheb_d0<<<g, kThreads, 0, st>>>(b, M.dinv, 1.0 / theta, dcur, n);
-        L->launches++;
+        k_cheb_d0<<<g, kThreads, 0, st>>>(b, W.dinv, P.c0, dcur, n);
+        p->launches++;
         rin = b;
         xmode = 2;                 // x = d0 + d1
     } else {
         SpmvEpi E;                 // r = b - A x ; d0 = dinv r / theta
-        E.b = b; E.dinv = M.dinv; E.rout = M.r; E.dout = dcur; E.c1 = 1.0 / theta;
-        if ((rc = mg_spmv_cheb(L, fp32, EPI_CHEB0, x, E))) return rc;
+        E.b = b; E.dinv = W.dinv; E.rout = W.r; E.dout = dcur; E.c1 = P.c0;
+        if ((rc = apply(EPI_CHEB0, x, E))) return rc;
         if (deg <= 1) {
             k_axpy<<<g, kThreads, 0, st>>>(1.0, dcur, x, n);
-            L->launches++;
+            p->launches++;
             FEMO_CHECK_LAUNCH();
             return FEMO_OK;
         }
-        rin = M.r;
+        rin = W.r;
         xmode = 1;                 // x += d0 + d1
     }
     for (int k = 2; k <= deg; ++k) {
-        const double rho_new = 1.0 / (2.0 * sigma - rho);
+        P.next();
         SpmvEpi E;
-        E.dinv = M.dinv; E.rin = rin; E.rout = M.r; E.dout = dnext; E.xacc = x;
-        E.c1 = rho_new * rho; E.c2 = 2.0 * rho_new / delta; E.xmode = xmode;
-        if (dia && k == deg) E.rout = E.dout = nullptr;      // nobody reads the last residual / direction
-        if ((rc = mg_spmv_cheb(L, fp32, EPI_CHEBK, dcur, E))) return rc;
+        E.dinv = W.dinv; E.rin = rin; E.rout = W.r; E.dout = dnext; E.xacc = x;
+        E.c1 = P.c1; E.c2 = P.c2; E.xmode = xmode;
+        if (drop_last && k == deg) E.rout = E.dout = nullptr;      // nobody reads the last residual / direction
+        if ((rc = apply(EPI_CHEBK, dcur, E))) return rc;
         std::swap(dcur, dnext);
-        rin = M.r;
+        rin = W.r;
         xmode = 0;
-        rho = rho_new;
     }
     return FEMO_OK;
 }
 
-struct MgParams {
-    int degree = 2;
-    double ratio = 4.0;
-    bool fp32 = true;      // V-cycle SpMVs stream fp32 copies of the level matrices (vectors stay fp64)
-};
+// the smoother of a geometric level; DIA levels add two shortcuts of k_dia_apply: the zero-guess degree-2 smoother as
+// one kernel, and no residual / direction stored by the last step (the kernel skips null outputs)
+static int mg_smooth(femo_problem *L, const double *b, double *x, bool zero_guess, int deg, double ratio, bool fp32) {
+    femo_mg_level &M = L->mgl;
+    const LevelOp op = level_op(L, fp32);
+    if (zero_guess && deg == 2 && op == LevelOp::DIA) {     // d0, the operator and both updates in one kernel
+        ChebPoly P(M.lmax, ratio);
+        P.next();
+        DiaEpi E;
+        E.b = b; E.c0 = P.c0; E.c1 = P.c1; E.c2 = P.c2;
+        return launch_dia(L, DIA_PRE2, nullptr, x, E);
+    }
+    return cheb_smooth(L, ChebWork{M.dinv, M.r, M.d, M.q, L->state.ndofs, M.lmax}, b, x, zero_guess, deg, ratio,
+                       op == LevelOp::DIA, [&](int kind, const double *xin, const SpmvEpi &E) {
+                           return level_apply(L, op, kind, xin, nullptr, E);
+                       });
+}
 
 static inline LatD latd_of(const femo_problem *p) {
     return LatD{p->mesh.n[0], p->mesh.n[1] + 1, p->slab.active ? p->slab.crow0 : 0};
@@ -936,7 +1007,7 @@ static int mgsweep_vcycle(femo_problem *root, int lv, const double *b, double *x
 // as one cooperative kernel (mgfused.cuh); single-GPU DIA levels above that range with a 2:1 nested coarse level run
 // their visit as two stencil sweeps (mgsweep.cuh); every other level takes the per-kernel path below.
 static int mg_vcycle(femo_problem *root, int lv, const double *b, double *x, const MgParams &mp) {
-    femo_problem *L = (lv == 0) ? root : root->mg[lv - 1];
+    femo_problem *L = mg_level(root, lv);
     const int nlev = (int)root->mg.size() + 1;
     femo_mg_level &M = L->mgl;
     const int64_t n = L->state.ndofs;
@@ -960,20 +1031,11 @@ static int mg_vcycle(femo_problem *root, int lv, const double *b, double *x, con
     }
     femo_problem *C = root->mg[lv];
     femo_mg_level &MC = C->mgl;
-    const DevPattern &D = L->dpat[0];
     if ((rc = mg_smooth(L, b, x, true, mp.degree, mp.ratio, mp.fp32))) return rc;
     // r = b - A x ; restrict
-    if (mp.fp32 && hex_matfree_ready(L)) {
-        SpmvEpi E;
-        E.b = b;
-        rc = launch_hex_matfree(L, EPI_PLAIN, x, M.r, E);
-    } else if (mp.fp32 && dia_ready(L)) {
-        DiaEpi E;
-        E.b = b;
-        rc = launch_dia(L, DIA_PLAIN, x, M.r, E);
-    } else if (mp.fp32 && M.vals32) rc = launch_spmv<false>(L, D.rb, D.nrb, D.rowptr, D.col, M.vals32, x, M.r, b, nullptr);
-    else rc = launch_spmv<false>(L, D.rb, D.nrb, D.rowptr, D.col, M.vals, x, M.r, b, nullptr);
-    if (rc) return rc;
+    SpmvEpi E;
+    E.b = b;
+    if ((rc = level_apply(L, level_op(L, mp.fp32), EPI_PLAIN, x, M.r, E))) return rc;
     if ((rc = mg_restrict(L, C, M.r, MC.b))) return rc;
     if ((rc = mg_vcycle(root, lv + 1, MC.b, MC.x, mp))) return rc;
     if ((rc = mg_prolong_add(L, C, MC.x, x))) return rc;
@@ -1044,23 +1106,20 @@ static int mg_prolong_add(femo_problem *L, femo_problem *C, double *xc, double *
     return FEMO_OK;
 }
 
-static int mg_vcycle(femo_problem *root, int lv, const double *b, double *x, const MgParams &mp);
-
 // Full-multigrid start (nested iteration): x0 ~ A^-1 b to discretisation accuracy for about 1.5 V-cycles
 // of work.  Coarsest level solved exactly; each finer level prolongs the coarser iterate and corrects
 // it with one V-cycle on its residual.
 static int mg_fmg(femo_problem *root, const double *b, double *x, const MgParams &mp) {
     const int nlev = (int)root->mg.size() + 1;
     int rc;
-    auto level = [&](int lv) { return lv == 0 ? root : root->mg[lv - 1]; };
     // right-hand sides of all levels
     for (int lv = 0; lv + 1 < nlev; ++lv) {
-        femo_problem *L = level(lv), *C = level(lv + 1);
+        femo_problem *L = mg_level(root, lv), *C = mg_level(root, lv + 1);
         double *rf = (lv == 0) ? const_cast<double *>(b) : L->mgl.fb;
         if ((rc = mg_restrict(L, C, rf, C->mgl.fb))) return rc;
     }
     for (int lv = nlev - 1; lv >= 0; --lv) {
-        femo_problem *L = level(lv);
+        femo_problem *L = mg_level(root, lv);
         femo_mg_level &M = L->mgl;
         const int64_t n = L->state.ndofs;
         cudaStream_t st = L->stream;
@@ -1071,20 +1130,21 @@ static int mg_fmg(femo_problem *root, const double *b, double *x, const MgParams
             L->launches++;
             continue;
         }
-        femo_problem *C = level(lv + 1);
+        femo_problem *C = mg_level(root, lv + 1);
         FEMO_CUDA(cudaMemsetAsync(xl, 0, sizeof(double) * n, st));
         if ((rc = mg_prolong_add(L, C, C->mgl.fx, xl))) return rc;
         // residual of the prolonged iterate into M.b (free at this level), V-cycle correction into M.x
-        const DevPattern &D = L->dpat[0];
         double *rl = (lv == 0) ? root->kr_r : M.b, *el = (lv == 0) ? root->kr_z : M.x;
-        // residual of the nested iterate: fp64 planes on the fine level, the V-cycle's fp32 planes below (the
-        // full-multigrid iterate is only the Krylov method's initial guess)
-        if (mp.fp32 && M.dia64_valid && dia_ready(L)) rc = launch_dia64<false>(L, xl, rl, bl, nullptr);
-        else if (mp.fp32 && dia_ready(L) && lv > 0) {
-            DiaEpi E;
+        // residual of the nested iterate: fp64 planes on the fine level, the V-cycle's fp32 planes below, fp64 CSR on
+        // every other level, matrix-free and CSR32 ones included (the full-multigrid iterate is only the Krylov
+        // method's initial guess)
+        const bool dia = level_op(L, mp.fp32) == LevelOp::DIA;
+        if (dia && M.dia64_valid) rc = launch_dia64<false>(L, xl, rl, bl, nullptr);
+        else {
+            SpmvEpi E;
             E.b = bl;
-            rc = launch_dia(L, DIA_PLAIN, xl, rl, E);
-        } else rc = launch_spmv<false>(L, D.rb, D.nrb, D.rowptr, D.col, M.vals, xl, rl, bl, nullptr);
+            rc = level_apply(L, dia && lv > 0 ? LevelOp::DIA : LevelOp::CSR64, EPI_PLAIN, xl, rl, E);
+        }
         if (rc) return rc;
         if ((rc = mg_vcycle(root, lv, rl, el, mp))) return rc;
         k_axpy<<<red_grid(L, n), kThreads, 0, st>>>(1.0, el, xl, n);
@@ -1106,7 +1166,7 @@ static int sync_replicated_bc(femo_problem *root) {
     while (g < root->mg.size() && !root->mg[g]->replicated) ++g;
     root->mg_bc_dirty = false;
     if (g == root->mg.size()) return FEMO_OK;
-    femo_problem *F = (g == 0) ? root : root->mg[g - 1];
+    femo_problem *F = mg_level(root, (int)g);
     femo_problem *C = root->mg[g];
     const int64_t nf = F->state.ndofs, nc = C->state.ndofs;
     cudaStream_t st = root->stream;
@@ -1141,7 +1201,7 @@ static int mg_setup(femo_problem *root, const double *vals, bool fp32 = true, bo
     if (root->mg_bc_dirty && (rc = sync_replicated_bc(root))) return rc;
     if (root->coef[0] && (rc = halo_nodes(root, const_cast<double *>(root->coef[0])))) return rc;
     for (int lv = 0; lv < nlev; ++lv) {
-        femo_problem *L = (lv == 0) ? root : root->mg[lv - 1];
+        femo_problem *L = mg_level(root, lv);
         femo_mg_level &M = L->mgl;
         cudaStream_t st = L->stream;
         const int64_t n = L->state.ndofs;
@@ -1149,7 +1209,7 @@ static int mg_setup(femo_problem *root, const double *vals, bool fp32 = true, bo
         if (lv == 0) {
             M.vals = const_cast<double *>(vals);
         } else {
-            femo_problem *F = (lv == 1) ? root : root->mg[lv - 2];
+            femo_problem *F = mg_level(root, lv - 1);
             const double *uf = (lv == 1) ? root->coef[0] : F->mgl.u;
             if (!uf) return set_err(FEMO_ESTATE, "multigrid setup: state coefficient not set");
             if (F->state.element == EL_P2) {                      // vertex values of the P2 state
@@ -1203,8 +1263,7 @@ static int mg_setup(femo_problem *root, const double *vals, bool fp32 = true, bo
                 L->coef[1] = M.m;
                 L->coefn[1] = ncell;
             }
-            DiaMat tmp;
-            direct = fp32 && lv < nlev - 1 && L->lattice_fast && M.vals32 && dia_offsets(L, tmp) && !g_env.no_lattice_asm;
+            direct = fp32 && lv < nlev - 1 && lattice_dia_direct(L);
             if (direct) rc = lattice_jacobian(L, nullptr, nullptr, true, L->has_bc);      // no CSR values on DIA-only levels
             else rc = femo_assemble_jacobian(L, L->has_bc ? nullptr : M.vals, L->has_bc ? M.vals : nullptr);
             if (rc) return rc;
