@@ -46,7 +46,7 @@ using namespace femo;
 
 struct AmgLevelDev {
     int64_t n = 0, nnz = 0, nc = 0, nnzP = 0, nnzAP = 0;
-    const int32_t *rowptr = nullptr, *col = nullptr, *rb = nullptr;
+    int32_t *rowptr = nullptr, *col = nullptr, *rb = nullptr;
     int nrb = 0;
     double *vals = nullptr;                 // level 0: the matrix of the current solve (not owned)
     double *dinv = nullptr, *x = nullptr, *b = nullptr, *r = nullptr, *d = nullptr, *q = nullptr;
@@ -64,80 +64,51 @@ struct femo_amg {
     AmgHier host;
     std::vector<AmgLevelDev> lv;
     bool attached = false;
-    size_t arena_bytes = 0;
+    size_t arena_bytes = 0;                 // counted by femo_amg_symbolic
     long long numeric_setups = 0;
 };
 
-// bytes of device memory the hierarchy needs (maps + values + work vectors of every level)
-static size_t amg_arena_bytes(const AmgHier &h) {
-    size_t w = 0;
+// The AMG arena's layout walk: maps, values and work vectors of every level, in level order.  Level 0 borrows the
+// problem's pattern.  femo_amg_symbolic runs it counting (Arena, common.cuh) to size the arena, femo_amg_attach placing.
+static void amg_lay_out(Arena &A, const femo_problem *p, const AmgHier &h, std::vector<AmgLevelDev> &lv) {
     const int nl = (int)h.lv.size();
+    lv.assign(nl, AmgLevelDev());
     for (int l = 0; l < nl; ++l) {
-        const AmgLevelHost &L = h.lv[l];
-        auto I = [&](size_t c) { w += Arena::need(std::max<size_t>(c, 1), 4); };
-        auto F = [&](size_t c) { w += Arena::need(std::max<size_t>(c, 1), 8); };
-        if (l > 0) { I(L.n + 1); I(L.nnz); I(L.rb.size()); F(L.nnz); }
-        F(L.n); F(L.n); F(L.n); F(L.n); F(L.n); F(L.n);                     // dinv, x, b, r, d, q
-        if (l + 1 < nl) {
-            I(L.n + 1); I(L.nnzP); I(L.nnzP); I(L.p_rb.size()); I(L.nnzP + 1); I(L.pp_src.size());
-            I(L.nc + 1); I(L.nnzP); I(L.nnzP); I(L.r_rb.size());
-            I(L.nnzAP + 1); I(L.ap_ia.size()); I(L.ap_ib.size());
-            I(L.nnzC + 1); I(L.ac_ia.size()); I(L.ac_ib.size());
-            F(L.nnzP); F(L.nnzP); F(L.nnzAP);
-        } else if (L.n <= kMgDenseMax) {
-            F((size_t)L.n * L.n); F((size_t)L.n * L.n);
-        }
-    }
-    return w + 4096;
-}
-
-static int amg_attach(femo_problem *p, femo_amg *G, void *d_arena, size_t bytes) {
-    Arena A;
-    A.reset(d_arena, bytes);
-    cudaStream_t st = p->stream;
-    const int nl = (int)G->host.lv.size();
-    G->lv.assign(nl, AmgLevelDev());
-    bool ok = true;
-    auto upI = [&](const std::vector<int32_t> &v) -> int32_t * {
-        int32_t *d = A.take<int32_t>(std::max<size_t>(v.size(), 1));
-        if (!d) { ok = false; return nullptr; }
-        if (!v.empty()) cudaMemcpyAsync(d, v.data(), v.size() * 4, cudaMemcpyHostToDevice, st);
-        return d;
-    };
-    auto F = [&](size_t c) -> double * {
-        double *d = A.take<double>(std::max<size_t>(c, 1));
-        if (!d) ok = false;
-        return d;
-    };
-    for (int l = 0; l < nl && ok; ++l) {
-        const AmgLevelHost &H = G->host.lv[l];
-        AmgLevelDev &L = G->lv[l];
+        const AmgLevelHost &H = h.lv[l];
+        AmgLevelDev &L = lv[l];
+        auto F = [&](double *&d, size_t c) { A.take(d, std::max<size_t>(c, 1)); };
         L.n = H.n; L.nnz = H.nnz; L.nc = H.nc; L.nnzP = H.nnzP; L.nnzAP = H.nnzAP;
         if (l == 0) {
             const DevPattern &D = p->dpat[0];
             L.rowptr = D.rowptr; L.col = D.col; L.rb = D.rb; L.nrb = D.nrb;
         } else {
-            L.rowptr = upI(H.rowptr); L.col = upI(H.col); L.rb = upI(H.rb); L.nrb = (int)H.rb.size() - 1;
-            L.vals = F(H.nnz);
+            put(A, L.rowptr, H.rowptr); put(A, L.col, H.col); put(A, L.rb, H.rb); L.nrb = (int)H.rb.size() - 1;
+            F(L.vals, H.nnz);
         }
-        L.dinv = F(H.n); L.x = F(H.n); L.b = F(H.n); L.r = F(H.n); L.d = F(H.n); L.q = F(H.n);
+        for (double **v : {&L.dinv, &L.x, &L.b, &L.r, &L.d, &L.q}) F(*v, H.n);
         if (l + 1 < nl) {
-            L.p_rowptr = upI(H.p_rowptr); L.p_col = upI(H.p_col); L.p_row = upI(H.p_row); L.p_rb = upI(H.p_rb);
+            put(A, L.p_rowptr, H.p_rowptr); put(A, L.p_col, H.p_col); put(A, L.p_row, H.p_row); put(A, L.p_rb, H.p_rb);
             L.p_nrb = (int)H.p_rb.size() - 1;
-            L.pp_ptr = upI(H.pp_ptr); L.pp_src = upI(H.pp_src);
-            L.r_rowptr = upI(H.r_rowptr); L.r_col = upI(H.r_col); L.r_perm = upI(H.r_perm); L.r_rb = upI(H.r_rb);
+            put(A, L.pp_ptr, H.pp_ptr); put(A, L.pp_src, H.pp_src);
+            put(A, L.r_rowptr, H.r_rowptr); put(A, L.r_col, H.r_col); put(A, L.r_perm, H.r_perm); put(A, L.r_rb, H.r_rb);
             L.r_nrb = (int)H.r_rb.size() - 1;
-            L.ap_ptr = upI(H.ap_ptr); L.ap_ia = upI(H.ap_ia); L.ap_ib = upI(H.ap_ib);
-            L.ac_ptr = upI(H.ac_ptr); L.ac_ia = upI(H.ac_ia); L.ac_ib = upI(H.ac_ib);
-            L.p_vals = F(H.nnzP); L.r_vals = F(H.nnzP); L.ap_vals = F(H.nnzAP);
+            put(A, L.ap_ptr, H.ap_ptr); put(A, L.ap_ia, H.ap_ia); put(A, L.ap_ib, H.ap_ib);
+            put(A, L.ac_ptr, H.ac_ptr); put(A, L.ac_ia, H.ac_ia); put(A, L.ac_ib, H.ac_ib);
+            F(L.p_vals, H.nnzP); F(L.r_vals, H.nnzP); F(L.ap_vals, H.nnzAP);
         } else if (H.n <= kMgDenseMax) {
-            L.dense = F((size_t)H.n * H.n); L.dense_tmp = F((size_t)H.n * H.n);
+            F(L.dense, (size_t)H.n * H.n); F(L.dense_tmp, (size_t)H.n * H.n);
         }
     }
-    FEMO_CUDA(cudaStreamSynchronize(st));
-    if (!ok) return set_err(FEMO_EINVAL, "femo_amg_attach: arena smaller than femo_amg_symbolic reported");
+}
+
+static int amg_attach(femo_problem *p, femo_amg *G, void *d_arena, size_t bytes) {
+    G->attached = false;
+    Arena A(d_arena, bytes, p->stream);
+    amg_lay_out(A, p, G->host, G->lv);
+    FEMO_CUDA(cudaStreamSynchronize(p->stream));
+    int rc = A.check(G->arena_bytes, "femo_amg_attach");
+    if (rc) return rc;
     G->attached = true;
-    G->arena_bytes = bytes;
     return FEMO_OK;
 }
 

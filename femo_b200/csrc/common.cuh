@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 
+#include <algorithm>
 #include <cstdint>
 #include <cstdio>
 #include <string>
@@ -105,20 +106,59 @@ struct DevVecMap {
     int32_t *ptr = nullptr, *src = nullptr;
 };
 
+// Bump allocator over a caller-provided device buffer, in 256-byte slots.  Each arena is filled by one layout walk that
+// runs in two modes.  An Arena without a buffer counts: take() only adds the rounded size to `used` and leaves its
+// destination alone, so the same walk is the size query and writes nothing.  With a buffer the walk places and uploads:
+// a take() that does not fit sets the sticky `failed` and hands out nullptr from then on, a failed copy is kept in
+// `err`, and the caller checks both once at the end (check()).
 struct Arena {
     char *base = nullptr;
     size_t cap = 0, used = 0;
-    void reset(void *b, size_t c) { base = (char *)b; cap = c; used = 0; }
+    cudaStream_t stream = nullptr;   // the copies of put / put_soa
+    bool failed = false;
+    cudaError_t err = cudaSuccess;
+    Arena() = default;
+    Arena(void *b, size_t c, cudaStream_t s = nullptr) : base((char *)b), cap(c), stream(s) {}
+    bool counting() const { return base == nullptr; }
     template <class T>
-    T *take(size_t count) {
-        size_t bytes = (count * sizeof(T) + 255) & ~size_t(255);
-        if (used + bytes > cap) return nullptr;
-        T *p = (T *)(base + used);
-        used += bytes;
-        return p;
+    void take(T *&dst, size_t count) {
+        const size_t at = used;
+        used += need(count, sizeof(T));
+        if (counting()) return;
+        failed |= used > cap;
+        dst = failed ? nullptr : (T *)(base + at);
+    }
+    void copy(void *dst, const void *src, size_t bytes) {
+        if (err == cudaSuccess) err = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyHostToDevice, stream);
+    }
+    // a placing walk succeeded: every copy was accepted and the layout took exactly the `counted` bytes of its count pass
+    int check(size_t counted, const std::string &what) const {
+        if (err != cudaSuccess) return set_err(FEMO_ECUDA, what + ": " + cudaGetErrorString(err));
+        if (failed || used != counted)
+            return set_err(FEMO_EINVAL, what + ": placed " + std::to_string(used) + " bytes, the size query counted " + std::to_string(counted));
+        return FEMO_OK;
     }
     static size_t need(size_t count, size_t elem) { return (count * elem + 255) & ~size_t(255); }
 };
+
+// reserve a host array's slot (at least one element) and copy the array in
+template <class T>
+void put(Arena &A, T *&dst, const std::vector<T> &src) {
+    A.take(dst, std::max<size_t>(1, src.size()));
+    if (!A.counting() && !A.failed && !src.empty()) A.copy(dst, src.data(), src.size() * sizeof(T));
+}
+// the same for an array of structures with `ncomp` components per entity, placed as ncomp planes (SoA)
+template <class T>
+void put_soa(Arena &A, T *&dst, const std::vector<T> &aos, int ncomp) {
+    A.take(dst, std::max<size_t>(1, aos.size()));
+    if (A.counting() || A.failed) return;
+    const size_t n = aos.size() / ncomp;
+    std::vector<T> soa(aos.size());
+    for (size_t e = 0; e < n; ++e)
+        for (int a = 0; a < ncomp; ++a) soa[a * n + e] = aos[e * ncomp + a];
+    if (!soa.empty()) A.copy(dst, soa.data(), soa.size() * sizeof(T));
+    if (A.err == cudaSuccess) A.err = cudaStreamSynchronize(A.stream);   // soa goes out of scope
+}
 
 // DIA (diagonal) storage of a lattice operator: nd planes of np fp32 values, plane s holds a(i, i + off[s]);
 // plane nd holds the Jacobi scaling (float)(1 / a_ii) used by every smoother step
@@ -213,7 +253,6 @@ struct femo_problem {
     cudaEvent_t ev_fork = nullptr, ev_join = nullptr;
     bool uploaded = false;
     int num_sms = 148;
-    femo::Arena st, wk;
     double *d_coords = nullptr;
     int32_t *d_cellsT = nullptr, *d_fb_cell = nullptr, *d_fb_local = nullptr, *d_cell_tag = nullptr;
     // P2 spaces: edge opposite each local vertex (SoA), edge -> vertices, vertex -> incident edges (CSR)

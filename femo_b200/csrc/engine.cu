@@ -538,21 +538,17 @@ static void hex_unit_stiffness(double hx, double hy, double hz, double nu, std::
 static bool hex_matfree_level(const femo_problem *p) {
     return p->family == FEMO_FAMILY_SIMP_HEX8 && p->mesh.kind == MESH_HEX && p->mesh.lattice && !getenv("FEMO_NO_MATFREE");
 }
-// upload K0 of this level's cells and reserve the cell-modulus array (arena: static for K0, work for ec)
-static int setup_hex_matfree(femo_problem *root, femo_problem *L) {
-    if (!hex_matfree_level(L)) return FEMO_OK;
+// layout walk of a matrix-free level (lay_out_problem): K0 of its cells in the static arena, the cell moduli in the work arena
+static void lay_out_matfree(femo_problem *L, Arena &st, Arena &wk) {
+    if (!hex_matfree_level(L)) return;
     const Mesh &M = L->mesh;
     const double hx = (M.hi[0] - M.lo[0]) / M.n[0], hy = (M.hi[1] - M.lo[1]) / M.n[1];
     const double hz = (M.hi[2] - M.lo[2]) / (double)(L->slab.active ? L->slab.gny : M.n[2]);
     std::vector<double> K;
     hex_unit_stiffness(hx, hy, hz, L->params[0], K);
-    L->h_k0 = K;
-    L->mgl.k0 = root->st.take<double>(576);
-    L->mgl.ec = root->wk.take<double>((size_t)M.ncells);
-    if (!L->mgl.k0 || !L->mgl.ec) return set_err(FEMO_EINVAL, "arena too small (matrix-free level)");
-    FEMO_CUDA(cudaMemcpyAsync(L->mgl.k0, K.data(), 576 * sizeof(double), cudaMemcpyHostToDevice, root->stream));
-    FEMO_CUDA(cudaStreamSynchronize(root->stream));
-    return FEMO_OK;
+    put(st, L->mgl.k0, K);
+    wk.take(L->mgl.ec, (size_t)M.ncells);
+    if (!st.counting()) L->h_k0 = std::move(K);   // the moved buffer stays alive for the pending copy
 }
 
 // the analytic-u_ex table of THIS problem into constant memory, stream-ordered before the kernel that reads it
@@ -876,15 +872,6 @@ static int read_scalars(femo_problem *p, int first, int count, double *h) {
     FEMO_CUDA(cudaMemcpyAsync(p->h_pinned, p->d_scalars + first, sizeof(double) * count, cudaMemcpyDeviceToHost, p->stream));
     FEMO_CUDA(cudaStreamSynchronize(p->stream));
     for (int i = 0; i < count; ++i) h[i] = p->h_pinned[i];
-    return FEMO_OK;
-}
-
-template <class T>
-static int up(femo_problem *p, T *&dst, const std::vector<T> &src) {
-    dst = p->st.take<T>(std::max<size_t>(1, src.size()));
-    if (!dst) return set_err(FEMO_EINVAL, "static arena too small");
-    if (!src.empty())
-        FEMO_CUDA(cudaMemcpyAsync(dst, src.data(), src.size() * sizeof(T), cudaMemcpyHostToDevice, p->stream));
     return FEMO_OK;
 }
 
@@ -1602,205 +1589,85 @@ int femo_problem_set_bc(femo_problem *p, const int32_t *dofs, const int32_t *lis
 }
 
 // ---- device residency -----------------------------------------------------
-static size_t pattern_bytes(const Pattern &P, bool bc) {
-    size_t b = 0;
-    b += Arena::need(P.rowptr.size(), 4) + Arena::need(P.col.size(), 4);
-    b += Arena::need(P.gptr.size(), 4) + Arena::need(P.gsrc.size(), 4);
-    b += Arena::need(P.t_rowptr.size(), 4) + Arena::need(P.t_col.size(), 4) + Arena::need(P.t_perm.size(), 4);
-    b += Arena::need(P.rb.size(), 4) + Arena::need(std::max<size_t>(1, P.t_rb.size()), 4);
-    if (bc) b += Arena::need(P.nnz, 1);
-    return b;
-}
-static size_t vecmap_bytes(const VecMap &V) { return Arena::need(V.ptr.size(), 4) + Arena::need(V.src.size(), 4); }
-
+// What the static and work arenas hold is decided in one place: the layout walk lay_out_problem, which covers the fine
+// level and then every coarse multigrid level (lay_out_level).  It runs twice (Arena, common.cuh): counting for
+// femo_problem_device_bytes and placing for femo_problem_upload, so the size query and the layout cannot disagree.  The
+// order of the reservations is the layout.  Host state derived while placing is set in place mode only, so the count
+// pass writes nothing into the problem.
 constexpr int kGmresRestart = 70;
 
-static void child_bytes(const femo_problem *c, bool coarsest, size_t *sb, size_t *wb) {
-    const Mesh &M = c->mesh;
-    const size_t N = (size_t)c->state.ndofs;
-    size_t s = 0, w = 0;
-    s += Arena::need(M.coords.size(), 8) + Arena::need(M.cells.size(), 4);
-    s += Arena::need(std::max<size_t>(1, c->fb_cell.size()), 4) * 2;
-    s += pattern_bytes(c->pat[0], true);
-    s += Arena::need(N, 1) + 2 * Arena::need(N, 8) + Arena::need(N, 4) + 1024;
-    if (hex_matfree_level(c)) { s += Arena::need(576, 8); w += Arena::need((size_t)c->mesh.ncells, 8); }
-    w += Arena::need(c->pat[0].nnz, 8) + Arena::need(fp32_copy_len(c), 4) + 9 * Arena::need(N, 8) + Arena::need((size_t)c->mesh.ncells, 8);
-    w += Arena::need(3 * kMaxPartials, 8) + Arena::need(S_COUNT, 8) + 1024;
-    if (coarsest) w += 2 * Arena::need(N * N, 8);
-    *sb = s;
-    *wb = w;
+// a matrix pattern (static): CSR, gather map, transpose permutation, SpMV row blocks, and the transposed CSR of a
+// rectangular pattern; a square pattern shares rowptr / col / row blocks with its transpose
+static void lay_out_pattern(Arena &st, const Pattern &P, DevPattern &D) {
+    put(st, D.rowptr, P.rowptr);
+    put(st, D.col, P.col);
+    put(st, D.gptr, P.gptr);
+    put(st, D.gsrc, P.gsrc);
+    put(st, D.t_perm, P.t_perm);
+    if (!P.square_symmetric) {
+        put(st, D.t_rowptr, P.t_rowptr);
+        put(st, D.t_col, P.t_col);
+    }
+    put(st, D.rb, P.rb);
+    if (!P.square_symmetric) put(st, D.t_rb, P.t_rb);
+    if (st.counting()) return;
+    D.nrb = (int)P.rb.size() - 1;
+    if (P.square_symmetric) {
+        D.t_rowptr = D.rowptr;
+        D.t_col = D.col;
+        D.t_rb = D.rb;
+        D.t_nrb = D.nrb;
+    } else {
+        D.t_nrb = (int)P.t_rb.size() - 1;
+    }
 }
 
-// place a coarse multigrid level in the root's arenas
-static int upload_child(femo_problem *root, femo_problem *c, bool coarsest) {
-    c->device = root->device;
-    c->stream = root->stream;
-    c->stream2 = root->stream2;
-    c->ev_fork = root->ev_fork;
-    c->ev_join = root->ev_join;
-    c->num_sms = root->num_sms;
+// Dirichlet arrays (static): per-nnz flag, marker, value, multiplicity, lifted rows.  Reserved with or without
+// conditions: femo_problem_set_bc may come after upload, and push_bc fills them.
+static void lay_out_bc(Arena &st, femo_problem *c) {
+    const int64_t N = c->state.ndofs;
+    st.take(c->dpat[0].bcflag, c->pat[0].nnz);
+    st.take(c->d_bc_mark, N);
+    st.take(c->d_bc_g, N);
+    st.take(c->d_bc_diag, N);
+    st.take(c->d_lift_rows, N);
+}
+
+// a coarse multigrid level in the root's arenas: mesh, Jacobian pattern and Dirichlet arrays (static); matrix values,
+// smoother and V-cycle vectors, and on the coarsest level the explicit inverse (work)
+static void lay_out_level(femo_problem *c, bool coarsest, Arena &st, Arena &wk) {
     const Mesh &M = c->mesh;
     const int64_t N = c->state.ndofs;
-    auto put = [&](auto *&dst, const auto &src) -> int {
-        using T = typename std::remove_reference<decltype(src)>::type::value_type;
-        dst = root->st.take<T>(std::max<size_t>(1, src.size()));
-        if (!dst) return set_err(FEMO_EINVAL, "static arena too small (multigrid level)");
-        if (!src.empty())
-            FEMO_CUDA(cudaMemcpyAsync(dst, src.data(), src.size() * sizeof(T), cudaMemcpyHostToDevice, root->stream));
-        return FEMO_OK;
-    };
-    int rc;
-    if ((rc = put(c->d_coords, M.coords))) return rc;
-    {
-        std::vector<int32_t> T(M.cells.size());
-        for (int64_t k = 0; k < M.ncells; ++k)
-            for (int a = 0; a < M.nvpc; ++a) T[a * M.ncells + k] = M.cells[k * M.nvpc + a];
-        if ((rc = put(c->d_cellsT, T))) return rc;
-        FEMO_CUDA(cudaStreamSynchronize(root->stream));
-    }
-    if ((rc = put(c->d_fb_cell, c->fb_cell))) return rc;
-    if ((rc = put(c->d_fb_local, c->fb_local))) return rc;
-    const Pattern &P = c->pat[0];
-    DevPattern &D = c->dpat[0];
-    if ((rc = put(D.rowptr, P.rowptr))) return rc;
-    if ((rc = put(D.col, P.col))) return rc;
-    if ((rc = put(D.gptr, P.gptr))) return rc;
-    if ((rc = put(D.gsrc, P.gsrc))) return rc;
-    if ((rc = put(D.t_perm, P.t_perm))) return rc;
-    if ((rc = put(D.rb, P.rb))) return rc;
-    D.nrb = (int)P.rb.size() - 1;
-    D.t_rowptr = D.rowptr; D.t_col = D.col; D.t_rb = D.rb; D.t_nrb = D.nrb;
-    D.bcflag = root->st.take<uint8_t>(P.nnz);
-    c->d_bc_mark = root->st.take<uint8_t>(N);
-    c->d_bc_g = root->st.take<double>(N);
-    c->d_bc_diag = root->st.take<double>(N);
-    c->d_lift_rows = root->st.take<int32_t>(N);
-    if (!c->d_lift_rows) return set_err(FEMO_EINVAL, "static arena too small (multigrid level)");
+    put(st, c->d_coords, M.coords);
+    put_soa(st, c->d_cellsT, M.cells, M.nvpc);
+    put(st, c->d_fb_cell, c->fb_cell);
+    put(st, c->d_fb_local, c->fb_local);
+    lay_out_pattern(st, c->pat[0], c->dpat[0]);
+    lay_out_bc(st, c);
     femo_mg_level &L = c->mgl;
-    L.vals = root->wk.take<double>(P.nnz);
-    L.vals32 = root->wk.take<float>(fp32_copy_len(c));
-    if ((rc = setup_hex_matfree(root, c))) return rc;
-    L.dinv = root->wk.take<double>(N);
-    L.x = root->wk.take<double>(N);
-    L.b = root->wk.take<double>(N);
-    L.r = root->wk.take<double>(N);
-    L.d = root->wk.take<double>(N);
-    L.q = root->wk.take<double>(N);
-    L.u = root->wk.take<double>(N);
-    L.m = root->wk.take<double>(std::max<int64_t>(1, c->mesh.ncells));
-    L.fb = root->wk.take<double>(N);
-    L.fx = root->wk.take<double>(N);
-    c->d_partials = root->wk.take<double>(3 * kMaxPartials);
-    c->d_scalars = root->wk.take<double>(S_COUNT);
-    if (c->d_scalars) FEMO_CUDA(cudaMemsetAsync(c->d_scalars, 0, sizeof(double) * S_COUNT, root->stream));
+    wk.take(L.vals, c->pat[0].nnz);
+    wk.take(L.vals32, fp32_copy_len(c));
+    lay_out_matfree(c, st, wk);
+    for (double **v : {&L.dinv, &L.x, &L.b, &L.r, &L.d, &L.q, &L.u}) wk.take(*v, N);
+    wk.take(L.m, std::max<int64_t>(1, M.ncells));
+    wk.take(L.fb, N);
+    wk.take(L.fx, N);
+    wk.take(c->d_partials, 3 * kMaxPartials);
+    wk.take(c->d_scalars, S_COUNT);
     if (coarsest) {
-        L.dense = root->wk.take<double>((size_t)N * N);
-        L.dense_tmp = root->wk.take<double>((size_t)N * N);
-        if (!L.dense_tmp) return set_err(FEMO_EINVAL, "work arena too small (multigrid level)");
+        wk.take(L.dense, (size_t)N * N);
+        wk.take(L.dense_tmp, (size_t)N * N);
     }
-    if (!c->d_scalars) return set_err(FEMO_EINVAL, "work arena too small (multigrid level)");
-    c->d_scratch = root->d_scratch;   // element tensors of coarse levels reuse the fine level's scratch
-    c->scratch_len = root->scratch_len;
-    if (!c->h_pinned) FEMO_CUDA(cudaMallocHost((void **)&c->h_pinned, sizeof(double) * 128));
-    if ((rc = push_bc(c))) return rc;
-    c->uploaded = true;
-    return FEMO_OK;
 }
 
-int femo_problem_device_bytes(const femo_problem *p, size_t *static_bytes, size_t *work_bytes) {
-    if (!p || !static_bytes || !work_bytes) return set_err(FEMO_EINVAL, "femo_problem_device_bytes: null");
-    refresh_env();
+static void lay_out_problem(femo_problem *p, Arena &st, Arena &wk) {
     const Mesh &M = p->mesh;
     const int64_t N = p->state.ndofs;
-    size_t s = 0;
-    s += Arena::need(M.coords.size(), 8) + Arena::need(M.cells.size(), 4);
-    s += 2 * Arena::need(std::max<size_t>(1, p->fb_cell.size()), 4) + Arena::need(std::max<size_t>(1, M.cell_tag.size()), 4);
-    s += Arena::need(2 * 49 * 4, 8);      // u_ex table
-    if (p->state.element == EL_P2)
-        s += Arena::need(M.cell_edges.size(), 4) + Arena::need(M.edge_verts.size(), 4) + Arena::need(p->vptr.size(), 4) + Arena::need(p->vedge.size(), 4);
-    if (p->state.element == EL_RMP) s += Arena::need(M.cell_edges.size(), 4);
-    for (int w = 0; w <= p->nin; ++w) s += pattern_bytes(p->pat[w], w == 0);
-    for (int m = 1; m < 4; ++m) s += vecmap_bytes(p->vm_state[m]);
-    for (int i = 0; i < p->nin; ++i) s += vecmap_bytes(p->vm_in[i]);
-    if (!p->pat[0].b_perm.empty())
-        s += Arena::need(p->pat[0].b_rowptr.size(), 4) + Arena::need(p->pat[0].b_col.size(), 4) +
-             Arena::need(p->pat[0].b_perm.size(), 4) + Arena::need(p->pat[0].b_rb.size(), 4);
-    s += Arena::need(N, 1) + 2 * Arena::need(N, 8) + Arena::need(N, 4);  // Dirichlet arrays (settable after upload)
-    s += 4096;
-    size_t scratch = 0, tv = 0;
-    for (int w = 0; w <= p->nin; ++w) {
-        scratch = std::max<size_t>(scratch, p->pat[w].scratch_len);
-        tv = std::max<size_t>(tv, p->pat[w].nnz);
-    }
-    for (int m = 1; m < 4; ++m) scratch = std::max<size_t>(scratch, p->vm_state[m].scratch_len);
-    for (int i = 0; i < p->nin; ++i) scratch = std::max<size_t>(scratch, p->vm_in[i].scratch_len);
-    scratch = std::max<size_t>(scratch, (size_t)M.ncells);
-    size_t w = 0;
-    w += Arena::need(scratch, 8);
-    w += Arena::need(3 * kMaxPartials, 8) + Arena::need(S_COUNT, 8);
-    w += 8 * Arena::need(N, 8);                    // r p q dinv z w b dx
-    w += 2 * Arena::need(p->pat[0].nnz, 8);        // Newton's Jacobian values (plain, BC'd)
-    w += Arena::need(tv, 8);                       // transposed values
-    if (!p->pat[0].b_perm.empty()) w += Arena::need(p->pat[0].nnz, 8);   // values as 3x3 blocks
-    w += Arena::need(N, 8);                        // Chebyshev direction of multigrid level 0
-    if (!p->mg.empty()) w += Arena::need(fp32_copy_len(p), 4);   // fp32 copy (CSR order or DIA planes)
-    if (!p->mg.empty()) w += Arena::need(kMgFusedMaxOps, sizeof(MgOp));   // op list of the cooperative coarse V-cycle
-    {
-        DiaMat A;
-        if (!p->mg.empty() && dia_offsets(p, A)) w += Arena::need((size_t)A.nd * (size_t)A.np, 8);   // fp64 planes (Krylov operator)
-    }
-    if (hex_matfree_level(p)) { s += Arena::need(576, 8); w += Arena::need((size_t)M.ncells, 8); }
-    if (N <= kMgDenseMax) w += 2 * Arena::need((size_t)N * N, 8);   // explicit inverse (precond 3)
-    if (!p->symmetric) w += (size_t)(kGmresRestart + 2) * Arena::need(N, 8) + Arena::need((size_t)(kGmresRestart + 1) * kMaxPartials, 8);
-    w += 4096;
-    for (size_t l = 0; l < p->mg.size(); ++l) {     // coarse multigrid levels live in the same arenas
-        size_t cs, cw;
-        child_bytes(p->mg[l], l + 1 == p->mg.size(), &cs, &cw);
-        s += cs;
-        w += cw;
-    }
-    *static_bytes = s;
-    *work_bytes = w;
-    return FEMO_OK;
-}
-
-int femo_problem_upload(femo_problem *p, int device, void *stream, void *d_static, size_t static_bytes, void *d_work,
-                        size_t work_bytes) {
-    if (!p || !d_static || !d_work) return set_err(FEMO_EINVAL, "femo_problem_upload: null");
-    if (femo_device_count() <= device || device < 0)
-        return set_err(FEMO_ENODEVICE, "femo_problem_upload: no such CUDA device; this engine has no CPU path");
-    size_t sb, wb;
-    femo_problem_device_bytes(p, &sb, &wb);
-    if (static_bytes < sb || work_bytes < wb) return set_err(FEMO_EINVAL, "femo_problem_upload: arenas smaller than femo_problem_device_bytes");
-    FEMO_CUDA(cudaSetDevice(device));
-    p->device = device;
-    p->stream = (cudaStream_t)stream;
-    cudaDeviceProp prop;
-    FEMO_CUDA(cudaGetDeviceProperties(&prop, device));
-    p->num_sms = prop.multiProcessorCount;
-    p->st.reset(d_static, static_bytes);
-    p->wk.reset(d_work, work_bytes);
-    if (!p->stream2) {
-        int lo_prio = 0, hi_prio = 0;
-        FEMO_CUDA(cudaDeviceGetStreamPriorityRange(&lo_prio, &hi_prio));
-        FEMO_CUDA(cudaStreamCreateWithPriority(&p->stream2, cudaStreamNonBlocking, hi_prio));
-        FEMO_CUDA(cudaEventCreateWithFlags(&p->ev_fork, cudaEventDisableTiming));
-        FEMO_CUDA(cudaEventCreateWithFlags(&p->ev_join, cudaEventDisableTiming));
-    }
-    const Mesh &M = p->mesh;
-    const int64_t N = p->state.ndofs;
-    int rc;
-    if ((rc = up(p, p->d_coords, M.coords))) return rc;
-    {   // cells as SoA planes
-        std::vector<int32_t> T(M.cells.size());
-        for (int64_t c = 0; c < M.ncells; ++c)
-            for (int a = 0; a < M.nvpc; ++a) T[a * M.ncells + c] = M.cells[c * M.nvpc + a];
-        if ((rc = up(p, p->d_cellsT, T))) return rc;
-        FEMO_CUDA(cudaStreamSynchronize(p->stream));  // T goes out of scope
-    }
-    if ((rc = up(p, p->d_fb_cell, p->fb_cell))) return rc;
-    if ((rc = up(p, p->d_fb_local, p->fb_local))) return rc;
-    if ((rc = up(p, p->d_cell_tag, M.cell_tag))) return rc;
+    put(st, p->d_coords, M.coords);
+    put_soa(st, p->d_cellsT, M.cells, M.nvpc);
+    put(st, p->d_fb_cell, p->fb_cell);
+    put(st, p->d_fb_local, p->fb_local);
+    put(st, p->d_cell_tag, M.cell_tag);
     if ((p->family == FEMO_FAMILY_NLPOISSON_P1 || p->family == FEMO_FAMILY_NLPOISSON_P2) && M.kind == MESH_TRI && M.lattice &&
         !p->jac_only && !getenv("FEMO_NO_UEX_TABLE")) {
         // u_ex = sin(2 pi x) sin(pi y) at x0 + dx_q: cos / sin of the offsets of the 49 points in both triangle types
@@ -1819,76 +1686,113 @@ int femo_problem_upload(femo_problem *p, int device, void *stream, void *d_stati
                     o[0] = std::cos(2.0 * pi * dx); o[1] = std::sin(2.0 * pi * dx);
                     o[2] = std::cos(pi * dy); o[3] = std::sin(pi * dy);
                 }
-        if ((rc = up(p, p->d_uex_tab, tab))) return rc;
-        FEMO_CUDA(cudaStreamSynchronize(p->stream));
-        p->h_uex_tab = tab;
+        put(st, p->d_uex_tab, tab);
+        if (!st.counting()) p->h_uex_tab = std::move(tab);   // the moved buffer stays alive for the pending copy
     }
-    if (p->state.element == EL_RMP) {
-        std::vector<int32_t> T(M.cell_edges.size());
-        for (int64_t c = 0; c < M.ncells; ++c)
-            for (int a = 0; a < 3; ++a) T[a * M.ncells + c] = M.cell_edges[c * 3 + a];
-        if ((rc = up(p, p->d_edgesT, T))) return rc;
-        FEMO_CUDA(cudaStreamSynchronize(p->stream));
-    }
+    if (p->state.element == EL_RMP || p->state.element == EL_P2) put_soa(st, p->d_edgesT, M.cell_edges, 3);
     if (p->state.element == EL_P2) {
-        std::vector<int32_t> T(M.cell_edges.size());
-        for (int64_t c = 0; c < M.ncells; ++c)
-            for (int a = 0; a < 3; ++a) T[a * M.ncells + c] = M.cell_edges[c * 3 + a];
-        if ((rc = up(p, p->d_edgesT, T))) return rc;
-        FEMO_CUDA(cudaStreamSynchronize(p->stream));
-        if ((rc = up(p, p->d_edge_verts, M.edge_verts))) return rc;
-        if ((rc = up(p, p->d_vptr, p->vptr))) return rc;
-        if ((rc = up(p, p->d_vedge, p->vedge))) return rc;
+        put(st, p->d_edge_verts, M.edge_verts);
+        put(st, p->d_vptr, p->vptr);
+        put(st, p->d_vedge, p->vedge);
     }
-    for (int w = 0; w <= p->nin; ++w) {
-        const Pattern &P = p->pat[w];
-        DevPattern &D = p->dpat[w];
-        if ((rc = up(p, D.rowptr, P.rowptr))) return rc;
-        if ((rc = up(p, D.col, P.col))) return rc;
-        if ((rc = up(p, D.gptr, P.gptr))) return rc;
-        if ((rc = up(p, D.gsrc, P.gsrc))) return rc;
-        if ((rc = up(p, D.t_perm, P.t_perm))) return rc;
-        if (P.square_symmetric) {
-            D.t_rowptr = D.rowptr;
-            D.t_col = D.col;
-        } else {
-            if ((rc = up(p, D.t_rowptr, P.t_rowptr))) return rc;
-            if ((rc = up(p, D.t_col, P.t_col))) return rc;
-        }
-        if ((rc = up(p, D.rb, P.rb))) return rc;
-        D.nrb = (int)P.rb.size() - 1;
-        if (P.square_symmetric) {
-            D.t_rb = D.rb;
-            D.t_nrb = D.nrb;
-        } else {
-            if ((rc = up(p, D.t_rb, P.t_rb))) return rc;
-            D.t_nrb = (int)P.t_rb.size() - 1;
-        }
-    }
+    for (int w = 0; w <= p->nin; ++w) lay_out_pattern(st, p->pat[w], p->dpat[w]);
     if (!p->pat[0].b_perm.empty()) {
         const Pattern &P = p->pat[0];
         DevPattern &D = p->dpat[0];
-        if ((rc = up(p, D.b_rowptr, P.b_rowptr))) return rc;
-        if ((rc = up(p, D.b_col, P.b_col))) return rc;
-        if ((rc = up(p, D.b_perm, P.b_perm))) return rc;
-        if ((rc = up(p, D.b_rb, P.b_rb))) return rc;
-        D.nbrb = (int)P.b_rb.size() - 1;
+        put(st, D.b_rowptr, P.b_rowptr);
+        put(st, D.b_col, P.b_col);
+        put(st, D.b_perm, P.b_perm);
+        put(st, D.b_rb, P.b_rb);
+        if (!st.counting()) D.nbrb = (int)P.b_rb.size() - 1;
     }
     for (int m = 1; m < 4; ++m) {
         if (p->vm_state[m].ptr.empty()) continue;
-        if ((rc = up(p, p->dvm_state[m].ptr, p->vm_state[m].ptr))) return rc;
-        if ((rc = up(p, p->dvm_state[m].src, p->vm_state[m].src))) return rc;
+        put(st, p->dvm_state[m].ptr, p->vm_state[m].ptr);
+        put(st, p->dvm_state[m].src, p->vm_state[m].src);
     }
     for (int i = 0; i < p->nin; ++i) {
-        if ((rc = up(p, p->dvm_in[i].ptr, p->vm_in[i].ptr))) return rc;
-        if ((rc = up(p, p->dvm_in[i].src, p->vm_in[i].src))) return rc;
+        put(st, p->dvm_in[i].ptr, p->vm_in[i].ptr);
+        put(st, p->dvm_in[i].src, p->vm_in[i].src);
     }
-    p->dpat[0].bcflag = p->st.take<uint8_t>(p->pat[0].nnz);
-    p->d_bc_mark = p->st.take<uint8_t>(N);
-    p->d_bc_g = p->st.take<double>(N);
-    p->d_bc_diag = p->st.take<double>(N);
-    p->d_lift_rows = p->st.take<int32_t>(N);
-    if (!p->d_lift_rows) return set_err(FEMO_EINVAL, "static arena too small");
+    lay_out_bc(st, p);
+
+    size_t scratch = 0, tv = 0;
+    for (int w = 0; w <= p->nin; ++w) {
+        scratch = std::max<size_t>(scratch, p->pat[w].scratch_len);
+        tv = std::max<size_t>(tv, p->pat[w].nnz);
+    }
+    for (int m = 1; m < 4; ++m) scratch = std::max<size_t>(scratch, p->vm_state[m].scratch_len);
+    for (int i = 0; i < p->nin; ++i) scratch = std::max<size_t>(scratch, p->vm_in[i].scratch_len);
+    scratch = std::max<size_t>(scratch, (size_t)M.ncells);
+    const int64_t nnz = p->pat[0].nnz;
+    wk.take(p->d_scratch, scratch);
+    wk.take(p->d_partials, 3 * kMaxPartials);
+    wk.take(p->d_scalars, S_COUNT);
+    for (double **v : {&p->kr_r, &p->kr_p, &p->kr_q, &p->kr_dinv, &p->kr_z, &p->kr_w, &p->nt_b, &p->nt_dx}) wk.take(*v, N);
+    wk.take(p->nt_vals, nnz);
+    wk.take(p->nt_vals_bc, nnz);
+    wk.take(p->d_tvals, tv);
+    if (!p->pat[0].b_perm.empty()) wk.take(p->d_bvals, nnz);
+    wk.take(p->kr_d, N);
+    if (!p->mg.empty()) {
+        wk.take(p->mgl.vals32, fp32_copy_len(p));
+        wk.take(p->d_mgops, kMgFusedMaxOps);
+        DiaMat A;   // fp64 planes of the fine-level operator for the Krylov recurrence (lattice stencil problems)
+        if (dia_offsets(p, A)) wk.take(p->mgl.dia64, (size_t)A.nd * (size_t)A.np);
+    }
+    lay_out_matfree(p, st, wk);
+    if (!p->symmetric) {   // GMRES: Krylov basis, a spare vector, multi-dot partials
+        wk.take(p->gm_basis, (size_t)(kGmresRestart + 1) * N);
+        wk.take(p->wk_extra, N);
+        wk.take(p->d_partials_big, (size_t)(kGmresRestart + 1) * kMaxPartials);
+    }
+    if (N <= kMgDenseMax) {   // explicit inverse (precond 3)
+        wk.take(p->d_dense, (size_t)N * N);
+        wk.take(p->d_dense_tmp, (size_t)N * N);
+    }
+    for (size_t l = 0; l < p->mg.size(); ++l) lay_out_level(p->mg[l], l + 1 == p->mg.size(), st, wk);
+    if (wk.counting()) return;
+    p->scratch_len = scratch;
+    p->tvals_len = tv;
+    if (!p->symmetric) p->gm_restart = kGmresRestart;
+}
+
+// both figures are exact: the count pass of the walk that femo_problem_upload places
+int femo_problem_device_bytes(const femo_problem *p, size_t *static_bytes, size_t *work_bytes) {
+    if (!p || !static_bytes || !work_bytes) return set_err(FEMO_EINVAL, "femo_problem_device_bytes: null");
+    refresh_env();
+    Arena st, wk;   // no buffers: the walk only counts, so *p stays as it is
+    lay_out_problem(const_cast<femo_problem *>(p), st, wk);
+    *static_bytes = st.used;
+    *work_bytes = wk.used;
+    return FEMO_OK;
+}
+
+int femo_problem_upload(femo_problem *p, int device, void *stream, void *d_static, size_t static_bytes, void *d_work,
+                        size_t work_bytes) {
+    if (!p || !d_static || !d_work) return set_err(FEMO_EINVAL, "femo_problem_upload: null");
+    if (femo_device_count() <= device || device < 0)
+        return set_err(FEMO_ENODEVICE, "femo_problem_upload: no such CUDA device; this engine has no CPU path");
+    size_t sb, wb;
+    femo_problem_device_bytes(p, &sb, &wb);
+    if (static_bytes < sb || work_bytes < wb) return set_err(FEMO_EINVAL, "femo_problem_upload: arenas smaller than femo_problem_device_bytes");
+    FEMO_CUDA(cudaSetDevice(device));
+    p->device = device;
+    p->stream = (cudaStream_t)stream;
+    cudaDeviceProp prop;
+    FEMO_CUDA(cudaGetDeviceProperties(&prop, device));
+    p->num_sms = prop.multiProcessorCount;
+    if (!p->stream2) {
+        int lo_prio = 0, hi_prio = 0;
+        FEMO_CUDA(cudaDeviceGetStreamPriorityRange(&lo_prio, &hi_prio));
+        FEMO_CUDA(cudaStreamCreateWithPriority(&p->stream2, cudaStreamNonBlocking, hi_prio));
+        FEMO_CUDA(cudaEventCreateWithFlags(&p->ev_fork, cudaEventDisableTiming));
+        FEMO_CUDA(cudaEventCreateWithFlags(&p->ev_join, cudaEventDisableTiming));
+    }
+    Arena st(d_static, static_bytes, p->stream), wk(d_work, work_bytes, p->stream);
+    lay_out_problem(p, st, wk);
+    int rc;
+    if ((rc = st.check(sb, "femo_problem_upload: static arena")) || (rc = wk.check(wb, "femo_problem_upload: work arena"))) return rc;
     if ((rc = push_bc(p))) return rc;
 
     // quadrature tables
@@ -1941,54 +1845,20 @@ int femo_problem_upload(femo_problem *p, int device, void *stream, void *d_stati
         FEMO_CUDA(cudaStreamSynchronize(p->stream));
     }
 
-    // work arena
-    size_t scratch = 0, tv = 0;
-    for (int w = 0; w <= p->nin; ++w) {
-        scratch = std::max<size_t>(scratch, p->pat[w].scratch_len);
-        tv = std::max<size_t>(tv, p->pat[w].nnz);
+    for (femo_problem *c : p->mg) {   // coarse levels run on the fine level's streams and reuse its element scratch
+        c->device = p->device;
+        c->stream = p->stream;
+        c->stream2 = p->stream2;
+        c->ev_fork = p->ev_fork;
+        c->ev_join = p->ev_join;
+        c->num_sms = p->num_sms;
+        c->d_scratch = p->d_scratch;
+        c->scratch_len = p->scratch_len;
+        FEMO_CUDA(cudaMemsetAsync(c->d_scalars, 0, sizeof(double) * S_COUNT, p->stream));
+        if (!c->h_pinned) FEMO_CUDA(cudaMallocHost((void **)&c->h_pinned, sizeof(double) * 128));
+        if ((rc = push_bc(c))) return rc;
+        c->uploaded = true;
     }
-    for (int m = 1; m < 4; ++m) scratch = std::max<size_t>(scratch, p->vm_state[m].scratch_len);
-    for (int i = 0; i < p->nin; ++i) scratch = std::max<size_t>(scratch, p->vm_in[i].scratch_len);
-    scratch = std::max<size_t>(scratch, (size_t)M.ncells);
-    p->scratch_len = scratch;
-    p->tvals_len = tv;
-    p->d_scratch = p->wk.take<double>(scratch);
-    p->d_partials = p->wk.take<double>(3 * kMaxPartials);
-    p->d_scalars = p->wk.take<double>(S_COUNT);
-    p->kr_r = p->wk.take<double>(N);
-    p->kr_p = p->wk.take<double>(N);
-    p->kr_q = p->wk.take<double>(N);
-    p->kr_dinv = p->wk.take<double>(N);
-    p->kr_z = p->wk.take<double>(N);
-    p->kr_w = p->wk.take<double>(N);
-    p->nt_b = p->wk.take<double>(N);
-    p->nt_dx = p->wk.take<double>(N);
-    p->nt_vals = p->wk.take<double>(p->pat[0].nnz);
-    p->nt_vals_bc = p->wk.take<double>(p->pat[0].nnz);
-    p->d_tvals = p->wk.take<double>(tv);
-    if (!p->pat[0].b_perm.empty()) p->d_bvals = p->wk.take<double>(p->pat[0].nnz);
-    p->kr_d = p->wk.take<double>(N);
-    if (!p->mg.empty()) p->mgl.vals32 = p->wk.take<float>(fp32_copy_len(p));
-    if (!p->mg.empty()) p->d_mgops = p->wk.take<MgOp>(kMgFusedMaxOps);
-    {   // fp64 planes of the fine-level operator for the Krylov recurrence (lattice stencil problems)
-        DiaMat A;
-        if (!p->mg.empty() && dia_offsets(p, A)) p->mgl.dia64 = p->wk.take<double>((size_t)A.nd * (size_t)A.np);
-    }
-    if ((rc = setup_hex_matfree(p, p))) return rc;
-    if (!p->symmetric) {
-        p->gm_restart = kGmresRestart;
-        p->gm_basis = p->wk.take<double>((size_t)(kGmresRestart + 1) * N);
-        p->wk_extra = p->wk.take<double>(N);
-        p->d_partials_big = p->wk.take<double>((size_t)(kGmresRestart + 1) * kMaxPartials);
-        if (!p->d_partials_big) return set_err(FEMO_EINVAL, "work arena too small (GMRES)");
-    }
-    if (N <= kMgDenseMax) {
-        p->d_dense = p->wk.take<double>((size_t)N * N);
-        p->d_dense_tmp = p->wk.take<double>((size_t)N * N);
-    }
-    if (!p->d_tvals || !p->kr_d) return set_err(FEMO_EINVAL, "work arena too small");
-    for (size_t l = 0; l < p->mg.size(); ++l)
-        if ((rc = upload_child(p, p->mg[l], l + 1 == p->mg.size()))) return rc;
     FEMO_CUDA(cudaMemsetAsync(p->d_scalars, 0, sizeof(double) * S_COUNT, p->stream));
     if (!p->h_pinned) FEMO_CUDA(cudaMallocHost((void **)&p->h_pinned, sizeof(double) * 128));
     FEMO_CUDA(cudaStreamSynchronize(p->stream));
@@ -2139,14 +2009,19 @@ int femo_problem_set_partition(femo_problem *p, int64_t n_owned_nodes, int64_t n
         return set_err(FEMO_EINVAL, "femo_problem_set_partition: owned + ghost nodes must cover the local mesh (owned first)");
     const int R = std::max(1, g_comm.nranks);
     const int64_t ns = n_send * b, ng = n_ghost * b, blk = std::max<int64_t>(1, blk_nodes * b);
-    const size_t need = Arena::need(std::max<int64_t>(ns, 1), 4) + Arena::need(std::max<int64_t>(ng, 1), 4) +
-                        Arena::need((size_t)blk * R, 8) + 1024;
+    GenPart &G = p->gpart;
+    auto lay_out = [&](Arena &A) {   // the buffer's layout walk: send indices, ghost sources, the gathered buffer of all ranks
+        A.take(G.d_send_idx, std::max<int64_t>(ns, 1));
+        A.take(G.d_ghost_src, std::max<int64_t>(ng, 1));
+        A.take(G.d_gather, (size_t)blk * R);
+    };
+    Arena count;
+    lay_out(count);
     if (!d_buf) {
-        *bytes = (int64_t)need;
+        *bytes = (int64_t)count.used;
         return FEMO_OK;
     }
-    if (*bytes < (int64_t)need) return set_err(FEMO_EINVAL, "femo_problem_set_partition: buffer smaller than the size query reported");
-    GenPart &G = p->gpart;
+    if (*bytes < (int64_t)count.used) return set_err(FEMO_EINVAL, "femo_problem_set_partition: buffer smaller than the size query reported");
     G.send_idx.resize(ns);
     G.ghost_src.resize(ng);
     for (int64_t k = 0; k < n_send; ++k) {
@@ -2161,12 +2036,8 @@ int femo_problem_set_partition(femo_problem *p, int64_t n_owned_nodes, int64_t n
     G.n_owned_dofs = n_owned_nodes * b;
     G.n_owned_cells = n_owned_cells;
     G.blk = blk;
-    Arena A;
-    A.reset(d_buf, (size_t)*bytes);
-    G.d_send_idx = A.take<int32_t>(std::max<int64_t>(ns, 1));
-    G.d_ghost_src = A.take<int32_t>(std::max<int64_t>(ng, 1));
-    G.d_gather = A.take<double>((size_t)blk * R);
-    if (!G.d_send_idx || !G.d_ghost_src || !G.d_gather) return set_err(FEMO_EINVAL, "femo_problem_set_partition: buffer too small");
+    Arena A(d_buf, (size_t)*bytes);
+    lay_out(A);
     FEMO_CUDA(cudaSetDevice(p->device));
     if (ns) FEMO_CUDA(cudaMemcpy(G.d_send_idx, G.send_idx.data(), ns * 4, cudaMemcpyHostToDevice));
     if (ng) FEMO_CUDA(cudaMemcpy(G.d_ghost_src, G.ghost_src.data(), ng * 4, cudaMemcpyHostToDevice));
@@ -2545,11 +2416,15 @@ int femo_amg_symbolic(femo_problem *p, const double *h_vals, const femo_amg_opts
         p->amg = nullptr;
         return set_err(e.code, e.msg);
     }
+    Arena count;
+    std::vector<AmgLevelDev> lv;
+    amg_lay_out(count, p, p->amg->host, lv);
+    p->amg->arena_bytes = count.used;
     if (info) {
         int64_t tot = 0;
         for (const AmgLevelHost &L : p->amg->host.lv) tot += L.nnz;
         info[0] = (int64_t)p->amg->host.lv.size();
-        info[1] = (int64_t)amg_arena_bytes(p->amg->host);
+        info[1] = (int64_t)p->amg->arena_bytes;
         info[2] = tot;
         info[3] = p->amg->host.lv.back().n;
     }
@@ -2560,7 +2435,7 @@ int femo_amg_attach(femo_problem *p, void *d_arena, int64_t bytes) {
     int rc;
     if ((rc = need_device(p))) return rc;
     if (!p->amg) return set_err(FEMO_ESTATE, "femo_amg_attach: run femo_amg_symbolic first");
-    if (!d_arena || bytes < (int64_t)amg_arena_bytes(p->amg->host)) return set_err(FEMO_EINVAL, "femo_amg_attach: arena too small");
+    if (!d_arena || bytes < (int64_t)p->amg->arena_bytes) return set_err(FEMO_EINVAL, "femo_amg_attach: arena too small");
     return amg_attach(p, p->amg, d_arena, (size_t)bytes);
 }
 

@@ -176,8 +176,11 @@ int femo_problem_mg_levels(const femo_problem *p);
 
 /* ---- device residency ------------------------------------------------------
  * Bytes the caller must provide: static (maps, patterns) and work (scratch,
- * Krylov vectors).  Upload copies the layout into d_static.  stream is a
- * cudaStream_t (NULL = legacy default stream). */
+ * Krylov vectors), for the problem and its multigrid levels.  Both figures are
+ * exact: the size query counts the same layout that upload places, and upload
+ * fails if the two ever differ.  Host only; no device is needed.  Upload copies
+ * the layout into d_static.  stream is a cudaStream_t (NULL = legacy default
+ * stream). */
 int femo_problem_device_bytes(const femo_problem *p, size_t *static_bytes, size_t *work_bytes);
 int femo_problem_upload(femo_problem *p, int device, void *stream, void *d_static, size_t static_bytes,
                         void *d_work, size_t work_bytes);
@@ -292,10 +295,10 @@ int femo_linear_solve(femo_problem *p, const double *d_vals, const double *d_b, 
  * patterns of P, R = P^T, A P, P^T A P on every level and the index lists of the numeric phase.  h_vals: host copy of
  * a (BC'd) Jacobian on the state pattern for the strength-of-connection test, or NULL (every connection strong).
  * Dirichlet rows (femo_problem_set_bc) are left out of the aggregates.  info[0] levels, info[1] bytes of device memory
- * femo_amg_attach needs, info[2] sum of nnz over the levels, info[3] dofs of the coarsest level.  femo_amg_attach
- * uploads the lists into the caller's buffer (a torch tensor, like the problem arenas).  The numeric phase (diagonals,
- * Gershgorin bounds, prolongator values, Galerkin products: sorted segmented reductions, no atomics) runs on the
- * device at the start of every precond-4 solve; femo_amg_numeric runs it alone. */
+ * femo_amg_attach needs (exact: the layout attach places, counted), info[2] sum of nnz over the levels, info[3] dofs of
+ * the coarsest level.  femo_amg_attach uploads the lists into the caller's buffer (a torch tensor, like the problem
+ * arenas).  The numeric phase (diagonals, Gershgorin bounds, prolongator values, Galerkin products: sorted segmented
+ * reductions, no atomics) runs on the device at the start of every precond-4 solve; femo_amg_numeric runs it alone. */
 typedef struct femo_amg_opts {
     double theta;        /* strength threshold |a_ij| >= theta sqrt(a_ii a_jj) on level 0 (default 0.08; < 0 keeps it) */
     double theta_decay;  /* factor per coarser level (default 0.5) */
