@@ -159,7 +159,7 @@ static int amg_numeric(femo_problem *p, femo_amg *G, const double *vals) {
             k_pair_segreduce<<<grid_for(C.nnz), kThreads, 0, st>>>(L.ac_ptr, L.ac_ia, L.ac_ib, L.p_vals, L.ap_vals, C.vals, C.nnz);
             p->launches += 4;
         } else if (L.dense) {
-            k_dense_inverse<<<1, kThreads, 0, st>>>(L.rowptr, L.col, L.vals, (int)L.n, L.dense_tmp, L.dense);
+            launch_dense_inverse(L.rowptr, L.col, L.vals, (int)L.n, L.dense_tmp, L.dense, st);
             p->launches++;
         }
         FEMO_CHECK_LAUNCH();

@@ -29,6 +29,9 @@ int set_err(int code, const std::string &msg);
 // linear scan of the environment and the solver enqueues a few thousand launches per step.
 struct EnvFlags {
     bool no_bsr = false, no_dia = false, no_overlap = false, no_mgfused = false, no_mgsweep = false, no_lattice_asm = false, no_graph = false, force_graph = false;
+    // A/B switches of the adjoint / set-up glue: FEMO_NO_TRANSPOSE_GATHER (transposed SpMV and adjoint DIA conversion through a permuted copy),
+    // FEMO_MG_SETUP_SYNC_EACH (one host read per multigrid level), FEMO_NO_BAND_INVERSE (Gauss-Jordan sweeps every row)
+    bool no_transpose_gather = false, mg_setup_sync_each = false, no_band_inverse = false;
     long long overlap_min_rows = 1 << 20, mgfused_max_rows = 20000, graph_max_rows = 1 << 20;
     long long mgfused_small_rows = 0;        // fused V-cycle ops up to this many rows run on ONE CTA (FEMO_MGFUSED_SMALL_ROWS); off:
                                              // measured slower (4096: 50.5 ms against 46.9 ms per step, profiles/r02_summary.md)
@@ -42,7 +45,8 @@ constexpr int kMaxPartials = 4096;   // upper bound on CTAs of any reducing kern
 constexpr int kMaxSlots = 12;
 
 // device scalar slots (doubles) used by the Krylov / Newton drivers
-enum Scalar { S_ALPHA = 0, S_BETA, S_RZ, S_RR, S_PQ, S_TMP0, S_TMP1, S_TMP2, S_BB, S_FLAG /* int flag raised by k_csr_to_dia */, S_GM = 16, S_COUNT = 128 };
+enum Scalar { S_ALPHA = 0, S_BETA, S_RZ, S_RR, S_PQ, S_TMP0, S_TMP1, S_TMP2, S_BB, S_FLAG /* int flag raised by k_csr_to_dia */, S_GM = 16,
+             S_MG = 96 /* multigrid set-up: S_TMP2..S_FLAG of each level, 3 slots per level */, S_COUNT = 128 };
 
 // ---- reductions (deterministic: fixed assignment, fixed tree) ---------------
 __device__ __forceinline__ double warp_sum(double v) {

@@ -32,6 +32,9 @@ void refresh_env() {
     g_env.no_mgsweep = getenv("FEMO_NO_MGSWEEP") != nullptr;
     g_env.no_lattice_asm = getenv("FEMO_NO_LATTICE_ASM") != nullptr;
     g_env.no_graph = getenv("FEMO_NO_GRAPH") != nullptr;
+    g_env.no_transpose_gather = getenv("FEMO_NO_TRANSPOSE_GATHER") != nullptr;
+    g_env.mg_setup_sync_each = getenv("FEMO_MG_SETUP_SYNC_EACH") != nullptr;
+    g_env.no_band_inverse = getenv("FEMO_NO_BAND_INVERSE") != nullptr;
     g_env.force_graph = getenv("FEMO_GRAPH") != nullptr;
     g_env.overlap_min_rows = num("FEMO_OVERLAP_MIN_ROWS", 1 << 20);
     g_env.mgfused_max_rows = num("FEMO_MGFUSED_MAX_ROWS", 20000);
@@ -200,11 +203,14 @@ __device__ __forceinline__ void spmv_row_epilogue(const SpmvEpi &E, int64_t i, d
     }
 }
 
-template <bool DOT, int EPI, class VT>
+// PERM: entry t of the row-block pattern has the value vals[vperm[t]] (a transposed product reads the untransposed values
+// through the pattern's t_perm instead of a permuted copy); the products and their sums are the same
+template <bool DOT, int EPI, class VT, bool PERM = false>
 __global__ void __launch_bounds__(kThreads)
     k_spmv(const int32_t *__restrict__ rb, int nrb, const int32_t *__restrict__ rowptr, const int32_t *__restrict__ col,
            const VT *__restrict__ vals, const double *__restrict__ x, double *__restrict__ y, SpmvEpi E,
-           double *__restrict__ partials) {
+           double *__restrict__ partials, const int32_t *__restrict__ vperm = nullptr) {
+    auto val = [&](int32_t t) -> double { return PERM ? (double)__ldg(vals + ld_stream(vperm + t)) : ld_stream(vals + t); };
     __shared__ double prod[kSpmvCap];
     __shared__ int32_t rp[kSpmvRows + 1];
     const int tid = threadIdx.x;
@@ -224,7 +230,7 @@ __global__ void __launch_bounds__(kThreads)
                 for (int j = 0; j < U; ++j) {
                     const int32_t t = base + j * kThreads;
                     c[j] = (t < e) ? ld_stream(col + t) : 0;
-                    v[j] = (t < e) ? ld_stream(vals + t) : 0.0;
+                    v[j] = (t < e) ? val(t) : 0.0;
                 }
 #pragma unroll
                 for (int j = 0; j < U; ++j) {
@@ -260,7 +266,7 @@ __global__ void __launch_bounds__(kThreads)
             }
         } else {  // a single long row: CTA-wide strided reduction (fixed order)
             double acc = 0.0;
-            for (int32_t t = s + tid; t < e; t += kThreads) acc += ld_stream(vals + t) * __ldg(x + ld_stream(col + t));
+            for (int32_t t = s + tid; t < e; t += kThreads) acc += val(t) * __ldg(x + ld_stream(col + t));
             acc = block_sum(acc);
             if (tid == 0) {
                 const double xi = __ldg(x + r0);
@@ -2301,6 +2307,13 @@ int femo_spmv(femo_problem *p, int which, const double *d_vals, const double *d_
         if ((rc = halo_nodes(p, const_cast<double *>(d_x)))) return rc;
     } else if ((rc = halo_cells(p, const_cast<double *>(d_x)))) return rc;
     if (!transpose) return launch_spmv<false>(p, D.rb, D.nrb, D.rowptr, D.col, d_vals, d_x, d_y, nullptr, nullptr, false);
+    if (!g_env.no_transpose_gather) {     // one pass: gather the values through t_perm
+        k_spmv<false, EPI_PLAIN, double, true><<<spmv_grid(p, D.t_nrb), kThreads, 0, p->stream>>>(
+            D.t_rb, D.t_nrb, D.t_rowptr, D.t_col, d_vals, d_x, d_y, SpmvEpi(), nullptr, D.t_perm);
+        p->launches++;
+        FEMO_CHECK_LAUNCH();
+        return FEMO_OK;
+    }
     k_permute<<<grid_for(P.nnz), kThreads, 0, p->stream>>>(D.t_perm, d_vals, p->d_tvals, P.nnz);
     p->launches++;
     FEMO_CHECK_LAUNCH();
@@ -2369,6 +2382,9 @@ int femo_linear_solve(femo_problem *p, const double *d_vals, const double *d_b, 
     memset(&o, 0, sizeof(o));
     if (opts) o = *opts;
     const double *vals = d_vals;
+    if (transpose && !g_env.no_transpose_gather && level0_dia_only(p, o)) {       // convert through t_perm, no copy
+        return cg_solve(p, d_vals, d_b, d_x, o, info, false, false, p->dpat[0].t_perm);
+    }
     if (transpose) {
         const int64_t nnz = p->pat[0].nnz;
         k_permute<<<grid_for(nnz), kThreads, 0, p->stream>>>(p->dpat[0].t_perm, d_vals, p->d_tvals, nnz);

@@ -50,6 +50,7 @@ __global__ void __launch_bounds__(kThreads) k_scale_to(double a, const double *_
 using namespace femo;
 
 constexpr int kGmresMax = 72;   // S_GM .. S_GM+kGmresMax scalar slots
+static_assert(S_GM + kGmresMax + 1 <= S_MG, "GMRES Hessenberg column overlaps the multigrid set-up slots");
 
 static int gmres_solve(femo_problem *p, const double *vals, const double *b, double *x, femo_krylov_opts o,
                        femo_krylov_info *info) {

@@ -243,7 +243,9 @@ static Precond precond_params(const femo_krylov_opts &o, ChebParams poly) {
 
 // set-up for the matrix `vals`.  q: the root's fourth V-cycle work vector (GMRES keeps kr_q for itself);
 // dia_prepared: `vals` was assembled with the fine level's DIA planes (mg_setup's level0_dia)
-static int precond_setup(femo_problem *p, const Precond &P, const double *vals, double *q, bool dia_prepared = false) {
+// vperm: the matrix is vals[vperm[t]] (multigrid only, see level0_dia_only)
+static int precond_setup(femo_problem *p, const Precond &P, const double *vals, double *q, bool dia_prepared = false,
+                         const int32_t *vperm = nullptr) {
     const int64_t n = p->state.ndofs;
     const DevPattern &D = p->dpat[0];
     cudaStream_t st = p->stream;
@@ -253,13 +255,15 @@ static int precond_setup(femo_problem *p, const Precond &P, const double *vals, 
     p->mgl.d = p->kr_d;
     p->mgl.q = q;
     if (P.pre == 2) {
-        if ((rc = mg_setup(p, vals, P.mg.fp32, dia_prepared))) return rc;
+        if ((rc = mg_setup(p, vals, P.mg.fp32, dia_prepared, vperm))) return rc;
+    } else if (vperm) {
+        return set_err(FEMO_ESTATE, "gathered values need the multigrid preconditioner");
     } else if (P.pre == 4) {
         if ((rc = amg_numeric(p, p->amg, vals))) return rc;
     } else if (P.pre == 1) {
         if ((rc = cheb_setup(p, vals))) return rc;
     } else if (P.pre == 3) {
-        k_dense_inverse<<<1, kThreads, 0, st>>>(D.rowptr, D.col, vals, (int)n, p->d_dense_tmp, p->d_dense);
+        launch_dense_inverse(D.rowptr, D.col, vals, (int)n, p->d_dense_tmp, p->d_dense, st);
         p->launches++;
     } else {
         k_diag_inv<<<grid_for(n), kThreads, 0, st>>>(D.rowptr, D.col, vals, p->kr_dinv, n);
@@ -290,7 +294,8 @@ static int precond_apply(femo_problem *p, const Precond &P, const double *in, do
 // problem (true inside femo_newton_solve, which assembles it itself): hexahedral lattices then apply the operator
 // matrix-free in the recurrence too.  Matrices handed in through femo_linear_solve are always streamed as given.
 static int cg_solve(femo_problem *p, const double *vals, const double *b, double *x, femo_krylov_opts o,
-                    femo_krylov_info *info, bool op_current = false, bool dia_prepared = false) {
+                    femo_krylov_info *info, bool op_current = false, bool dia_prepared = false,
+                    const int32_t *vperm = nullptr) {
     default_krylov(o);
     if (o.precond == 2 && p->mg.empty()) o.precond = 0;
     if (o.precond == 3 && !p->d_dense) return set_err(FEMO_ELIMIT, "precond 3 (dense direct) needs N <= 512 on one GPU");
@@ -306,7 +311,7 @@ static int cg_solve(femo_problem *p, const double *vals, const double *b, double
     double *pa = p->d_partials, *pb = p->d_partials + kMaxPartials;
     const int g = red_grid(p, n), go = red_grid(p, p->own_n);
     int rc, np = 0, spmvs = 0;
-    if ((rc = precond_setup(p, P, vals, p->kr_q, dia_prepared))) return rc;
+    if ((rc = precond_setup(p, P, vals, p->kr_q, dia_prepared, vperm))) return rc;
     // ||b||^2
     k_dot<<<go, kThreads, 0, st>>>(b + p->own_off, b + p->own_off, p->own_n, pa);
     p->launches++;
@@ -318,6 +323,7 @@ static int cg_solve(femo_problem *p, const double *vals, const double *b, double
     const bool mf_outer = op_current && pre == 2 && vop == LevelOp::MATFREE;
     const bool dia_outer = pre == 2 && p->mgl.dia64_valid && vop == LevelOp::DIA;       // fp64 planes of `vals` (set-up)
     const bool bsr_outer = !mf_outer && !dia_outer && bsr3_ready(p);                     // vector states in 3-D: 3x3 blocks
+    if (vperm && !dia_outer) return set_err(FEMO_ESTATE, "gathered values need the fp64 DIA planes for the recurrence");
     if (bsr_outer && (rc = bsr3_convert(p, vals))) return rc;
     // q = A xin with the recurrence's operator; dot = std::true_type: also the partial sums of xin.q, their count into np
     auto outer = [&](auto dot, const double *xin, double *q) -> int {

@@ -487,36 +487,41 @@ __global__ void __launch_bounds__(kThreads)
     }
 }
 
-// one CTA: dense inverse of a small CSR matrix by Gauss-Jordan with partial pivoting
-__global__ void __launch_bounds__(kThreads)
+// one CTA: dense inverse of a small CSR matrix by Gauss-Jordan with partial pivoting.  BAND: 1024 threads, each step
+// updates only the rows with a nonzero multiplier (see below); the pivots and the inverse are the same doubles as the full
+// sweep (!BAND, 256 threads), whose pivot search picks the same row at any thread count (ties go to the lower index).
+template <bool BAND, int NT = BAND ? 1024 : kThreads>
+__global__ void __launch_bounds__(NT)
     k_dense_inverse(const int32_t *__restrict__ rowptr, const int32_t *__restrict__ col, const double *__restrict__ vals,
                     int n, double *__restrict__ A, double *__restrict__ Inv) {
     __shared__ double fac[kMgDenseMax];
-    __shared__ int piv;
+    __shared__ int rows[BAND ? kMgDenseMax : 1];
+    __shared__ int piv, nrows;
+    __shared__ double rowA[BAND ? kMgDenseMax : 1], rowI[BAND ? kMgDenseMax : 1];   // the normalised pivot row
     const int tid = threadIdx.x;
-    for (int idx = tid; idx < n * n; idx += kThreads) {
+    for (int idx = tid; idx < n * n; idx += NT) {
         A[idx] = 0.0;
         Inv[idx] = (idx / n == idx % n) ? 1.0 : 0.0;
     }
     __syncthreads();
-    for (int i = tid; i < n; i += kThreads)
+    for (int i = tid; i < n; i += NT)
         for (int32_t t = rowptr[i]; t < rowptr[i + 1]; ++t) A[i * n + col[t]] = vals[t];
     __syncthreads();
-    __shared__ double pvv[kThreads];
-    __shared__ int pvi[kThreads];
+    __shared__ double pvv[NT];
+    __shared__ int pvi[NT];
     for (int k = 0; k < n; ++k) {
         // pivot = first row of maximal |A[i][k]|, i >= k: block-wide argmax (ties to the lower index, as a serial scan would)
         {
             double bv = -1.0;
             int best = k;
-            for (int i = k + tid; i < n; i += kThreads) {
+            for (int i = k + tid; i < n; i += NT) {
                 const double v = fabs(A[i * n + k]);
                 if (v > bv) { bv = v; best = i; }
             }
             pvv[tid] = bv;
             pvi[tid] = best;
             __syncthreads();
-            for (int o = kThreads / 2; o > 0; o >>= 1) {
+            for (int o = NT / 2; o > 0; o >>= 1) {
                 if (tid < o) {
                     const double v2 = pvv[tid + o];
                     const int i2 = pvi[tid + o];
@@ -529,29 +534,63 @@ __global__ void __launch_bounds__(kThreads)
         __syncthreads();
         const int pr = piv;
         if (pr != k)
-            for (int j = tid; j < n; j += kThreads) {
+            for (int j = tid; j < n; j += NT) {
                 double t = A[k * n + j]; A[k * n + j] = A[pr * n + j]; A[pr * n + j] = t;
                 t = Inv[k * n + j]; Inv[k * n + j] = Inv[pr * n + j]; Inv[pr * n + j] = t;
             }
         __syncthreads();
         const double pv = 1.0 / A[k * n + k];
         __syncthreads();
-        for (int j = tid; j < n; j += kThreads) {
-            A[k * n + j] *= pv;
-            Inv[k * n + j] *= pv;
+        for (int j = tid; j < n; j += NT) {
+            const double a = A[k * n + j] * pv, v = Inv[k * n + j] * pv;
+            A[k * n + j] = a;
+            Inv[k * n + j] = v;
+            if (BAND) { rowA[j] = a; rowI[j] = v; }
         }
-        for (int i = tid; i < n; i += kThreads) fac[i] = (i == k) ? 0.0 : A[i * n + k];
-        __syncthreads();
-        for (int idx = tid; idx < n * n; idx += kThreads) {
-            const int i = idx / n, j = idx % n;
-            const double f = fac[i];
-            if (f != 0.0) {
-                A[idx] -= f * A[k * n + j];
-                Inv[idx] -= f * Inv[k * n + j];
+        if (BAND) {
+            // only the rows with a nonzero multiplier change: list them (in any order, their updates are independent) and
+            // sweep each one warp-wide, the same update of the same entries as the full sweep below.  On a lattice coarse
+            // level that is the band below the pivot plus the filled rows above it, about half the rows.  Columns <= k of
+            // A are never read again (every later read of A is in a column > k), so A is updated right of the pivot only;
+            // Inv over all n columns.
+            if (tid == 0) nrows = 0;
+            __syncthreads();
+            for (int i = tid; i < n; i += NT) {
+                const double f = (i == k) ? 0.0 : A[i * n + k];
+                if (f != 0.0) {
+                    fac[i] = f;
+                    rows[atomicAdd(&nrows, 1)] = i;
+                }
+            }
+            __syncthreads();
+            const int warp = tid >> 5, lane = tid & 31, nr = nrows;
+            for (int r = warp; r < nr; r += NT / 32) {
+                const int i = rows[r];
+                const double f = fac[i];
+                for (int j = k + 1 + lane; j < n; j += 32) A[i * n + j] -= f * rowA[j];
+                for (int j = lane; j < n; j += 32) Inv[i * n + j] -= f * rowI[j];
+            }
+        } else {
+            for (int i = tid; i < n; i += NT) fac[i] = (i == k) ? 0.0 : A[i * n + k];
+            __syncthreads();
+            for (int idx = tid; idx < n * n; idx += NT) {
+                const int i = idx / n, j = idx % n;
+                const double f = fac[i];
+                if (f != 0.0) {
+                    A[idx] -= f * A[k * n + j];
+                    Inv[idx] -= f * Inv[k * n + j];
+                }
             }
         }
         __syncthreads();
     }
+}
+
+// coarsest-level inverse: the row-compacted sweep unless FEMO_NO_BAND_INVERSE asks for the full one
+static inline void launch_dense_inverse(const int32_t *rowptr, const int32_t *col, const double *vals, int n, double *A,
+                                        double *Inv, cudaStream_t st) {
+    if (g_env.no_band_inverse) k_dense_inverse<false><<<1, kThreads, 0, st>>>(rowptr, col, vals, n, A, Inv);
+    else k_dense_inverse<true><<<1, 1024, 0, st>>>(rowptr, col, vals, n, A, Inv);
 }
 
 // x = Inv * b (tiny system: one warp per row)
@@ -752,8 +791,9 @@ static inline size_t fp32_copy_len(const femo_problem *L) {
     return n;
 }
 
-// re-layout the level's assembled (BC'd) values as DIA planes in the fp32 buffer
-static int dia_convert(femo_problem *L) {
+// re-layout the level's assembled (BC'd) values as DIA planes in the fp32 buffer; vperm: the level's values are
+// M.vals[vperm[t]] (the transpose of M.vals through the square pattern's t_perm)
+static int dia_convert(femo_problem *L, const int32_t *vperm = nullptr) {
     femo_mg_level &M = L->mgl;
     DiaMat A;
     if (!dia_offsets(L, A) || !M.vals32) return FEMO_OK;
@@ -763,9 +803,14 @@ static int dia_convert(femo_problem *L) {
     const int g = grid_for(A.n);
     double *part = L->d_scratch ? L->d_scratch : L->d_partials;      // per-CTA maxima: the element scratch is free here
     if ((size_t)g > L->scratch_len) return set_err(FEMO_ESTATE, "DIA conversion: scratch too small for the partial maxima");
-    k_csr_to_dia<7><<<g, kThreads, 0, L->stream>>>(D.rowptr, D.col, M.vals, A, M.vals32,
-                                                   reinterpret_cast<int *>(L->d_scalars + S_FLAG), M.dinv, L->own_off,
-                                                   L->own_off + L->own_n, part, M.dia64);
+    if (vperm)
+        k_csr_to_dia<7, true><<<g, kThreads, 0, L->stream>>>(D.rowptr, D.col, M.vals, A, M.vals32,
+                                                             reinterpret_cast<int *>(L->d_scalars + S_FLAG), M.dinv,
+                                                             L->own_off, L->own_off + L->own_n, part, M.dia64, vperm);
+    else
+        k_csr_to_dia<7><<<g, kThreads, 0, L->stream>>>(D.rowptr, D.col, M.vals, A, M.vals32,
+                                                       reinterpret_cast<int *>(L->d_scalars + S_FLAG), M.dinv, L->own_off,
+                                                       L->own_off + L->own_n, part, M.dia64);
     M.dia64_valid = M.dia64 != nullptr;
     k_max_finalize<<<1, kThreads, 0, L->stream>>>(part, g, L->d_scalars, S_TMP2);
     L->launches += 2;
@@ -1191,15 +1236,47 @@ static int sync_replicated_bc(femo_problem *root) {
     return propagate_bc(root, (int)g + 1);
 }
 
+// A CG solve with the fp32 geometric multigrid reads the fine level's CSR values only through its DIA conversion when
+// the fine level converts (mg_setup's DIA branch: lattice P1, fp32 and fp64 planes, not the coarsest level): the V-cycle
+// streams the fp32 planes, the recurrence and the full-multigrid residual the fp64 planes.  Then a transposed solve can
+// convert through the pattern's t_perm instead of permuting every value first.
+static bool level0_dia_only(const femo_problem *p, const femo_krylov_opts &o) {
+    DiaMat A;
+    return o.method == 0 && o.precond == 2 && o.mg_precision == 0 && !p->mg.empty() && p->dpat[0].t_perm &&
+           !hex_matfree_ready(p) && p->mgl.vals32 && p->mgl.dia64 && dia_offsets(p, A);
+}
+
 // (re)build the hierarchy for the matrix `vals` of the root at the root's current state
 // level0_dia: the caller has just assembled `vals` with lattice_jacobian(..., with_dia = true): the fine level's DIA
 // planes, dinv and Gershgorin maximum are already in place
-static int mg_setup(femo_problem *root, const double *vals, bool fp32 = true, bool level0_dia = false) {
+// vperm: the fine level's matrix is vals[vperm[t]] (see level0_dia_only); only its DIA conversion may read `vals`
+static int mg_setup(femo_problem *root, const double *vals, bool fp32 = true, bool level0_dia = false,
+                    const int32_t *vperm = nullptr) {
     if (root->mg.empty()) return set_err(FEMO_ESTATE, "multigrid requested but femo_problem_enable_multigrid was not called before upload");
+    if (vperm && level0_dia) return set_err(FEMO_ESTATE, "multigrid setup: gathered values cannot come with DIA planes");
     const int nlev = (int)root->mg.size() + 1;
     int rc;
     if (root->mg_bc_dirty && (rc = sync_replicated_bc(root))) return rc;
     if (root->coef[0] && (rc = halo_nodes(root, const_cast<double *>(root->coef[0])))) return rc;
+    // Every level's Gershgorin bound and DIA error flag (its S_TMP2 .. S_FLAG) is copied into the root's S_MG slots on the
+    // stream, and all of them come to the host in one read once every level is enqueued.  No level's set-up reads a
+    // host-side lmax: only the smoothers and the fused coarse program use it, and they run after the set-up.
+    constexpr int kSlots = S_FLAG - S_TMP2 + 1, kBatch = (S_COUNT - S_MG) / kSlots;
+    femo_problem *pend[kBatch];
+    int npend = 0;
+    auto flush = [&]() -> int {
+        if (!npend) return FEMO_OK;
+        double lm[kBatch * kSlots];
+        int rc2 = read_scalars(root, S_MG, npend * kSlots, lm);
+        if (rc2) return rc2;
+        for (int j = 0; j < npend; ++j) {
+            pend[j]->mgl.lmax = lm[j * kSlots];
+            if (lm[j * kSlots + S_FLAG - S_TMP2] != 0.0)
+                return set_err(FEMO_ESTATE, "DIA conversion met a column offset outside the lattice stencil");
+        }
+        npend = 0;
+        return FEMO_OK;
+    };
     for (int lv = 0; lv < nlev; ++lv) {
         femo_problem *L = mg_level(root, lv);
         femo_mg_level &M = L->mgl;
@@ -1277,8 +1354,10 @@ static int mg_setup(femo_problem *root, const double *vals, bool fp32 = true, bo
             k_pow_cells<<<grid_for(ncell), kThreads, 0, st>>>(L->coef[1], L->params[4], M.ec, ncell);
             L->launches++;
         } else if (fp32 && M.vals32 && lv < nlev - 1 && dia_offsets(L, M.dia)) {
-            if ((rc = dia_convert(L))) return rc;
+            if ((rc = dia_convert(L, lv == 0 ? vperm : nullptr))) return rc;
             dia_setup = true;
+        } else if (lv == 0 && vperm) {
+            return set_err(FEMO_ESTATE, "multigrid setup: gathered fine-level values need its DIA conversion");
         } else if (fp32 && M.vals32 && lv < nlev - 1) {
             M.dia_valid = false;
             M.dia64_valid = false;
@@ -1288,7 +1367,7 @@ static int mg_setup(femo_problem *root, const double *vals, bool fp32 = true, bo
         }
         if (lv == nlev - 1) {
             if (n > kMgDenseMax) return set_err(FEMO_ELIMIT, "multigrid: coarsest level too large for the dense solve");
-            k_dense_inverse<<<1, kThreads, 0, st>>>(D.rowptr, D.col, M.vals, (int)n, M.dense_tmp, M.dense);
+            launch_dense_inverse(D.rowptr, D.col, M.vals, (int)n, M.dense_tmp, M.dense, st);
             L->launches++;
         } else {
             if (!dia_setup) {
@@ -1299,13 +1378,14 @@ static int mg_setup(femo_problem *root, const double *vals, bool fp32 = true, bo
                 FEMO_CHECK_LAUNCH();
             }
             if ((rc = allreduce_scalars(L, S_TMP2, 1, true))) return rc;
-            double lm[3];
-            if ((rc = read_scalars(L, S_TMP2, 3, lm))) return rc;
-            M.lmax = lm[0];
-            if (lm[2] != 0.0) return set_err(FEMO_ESTATE, "DIA conversion met a column offset outside the lattice stencil");
+            FEMO_CUDA(cudaMemcpyAsync(root->d_scalars + S_MG + npend * kSlots, L->d_scalars + S_TMP2, sizeof(double) * kSlots,
+                                      cudaMemcpyDeviceToDevice, st));
+            pend[npend++] = L;
+            if ((npend == kBatch || g_env.mg_setup_sync_each) && (rc = flush())) return rc;
         }
         FEMO_CHECK_LAUNCH();
     }
+    if ((rc = flush())) return rc;
     root->mgprog.dirty = true;       // level bounds changed: the fused coarse V-cycle program is rebuilt on first use
     return FEMO_OK;
 }

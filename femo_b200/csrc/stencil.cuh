@@ -24,11 +24,14 @@ namespace femo {
 // entry's offset is not in the table (the host checked the pattern, so this never fires on a sane layout).
 // The same pass yields what the smoother set-up needs from the fp64 values: dinv_i = 1/a_ii and the per-CTA maximum of
 // the Gershgorin bound sum_j |a_ij| / |a_ii| over the owned rows [o0,o1) (partials[blockIdx.x]).
-template <int D>
+// PERM: entry t has the value vals[vperm[t]]; with a square pattern's t_perm that converts the transpose without a
+// permuted copy (same values in the same order, so the same planes, dinv and bound as converting the copy).
+template <int D, bool PERM = false>
 __global__ void __launch_bounds__(kThreads)
     k_csr_to_dia(const int32_t *__restrict__ rowptr, const int32_t *__restrict__ col, const double *__restrict__ vals,
                  DiaMat A, float *__restrict__ planes, int *__restrict__ bad, double *__restrict__ dinv, int64_t o0,
-                 int64_t o1, double *__restrict__ partials, double *__restrict__ planes64) {
+                 int64_t o1, double *__restrict__ partials, double *__restrict__ planes64,
+                 const int32_t *__restrict__ vperm = nullptr) {
     const int64_t i = blockIdx.x * (int64_t)blockDim.x + threadIdx.x;
     double g = 0.0;
     if (i < A.n) {
@@ -39,7 +42,7 @@ __global__ void __launch_bounds__(kThreads)
         double diag = 1.0, sabs = 0.0;
         for (int32_t t = rowptr[i]; t < rowptr[i + 1]; ++t) {
             const int d = col[t] - (int)i;
-            const double v64 = vals[t];
+            const double v64 = PERM ? __ldg(vals + __ldg(vperm + t)) : vals[t];
             const float v = (float)v64;
             sabs += fabs(v64);
             if (d == 0) diag = v64;
