@@ -26,10 +26,16 @@
 
 namespace femo {
 
-constexpr int kSwThreads = 256;                  // one thread per tile column
+// A CTA retires one row per iteration between two barriers, and a row's instructions (address and range arithmetic,
+// conversions, two dependent fp64 stencil chains) keep the issue slots of an SM busy: the sweeps run at the pace of
+// the rows the resident CTAs have in progress, not at that of the loads in flight.  Tiles of 128 threads put 8 (down) /
+// 6 (up) CTAs on an SM with half as many warps behind each barrier as 256-thread tiles, and bands may be one coarse
+// row high, so that the levels of 63 k - 1 M rows, which a wave of 8-row bands could not fill, spread over every SM.
+// Measured on a B200 (1000 W, n = 4000): 37.27 ms per bench step against 38.83 ms with 256-thread tiles and 8-row bands.
+constexpr int kSwThreads = 128;                  // one thread per tile column
 constexpr int kSwHalo = 3;                       // halo columns per side
 constexpr int kSwMaxCols = kSwThreads - 2 * kSwHalo;
-constexpr int kSwMinRows = 8;                    // coarse rows per CTA at least (the band's warm-up is 4 coarse rows)
+constexpr int kSwMinRows = 1;                    // coarse rows per CTA at least (a band also computes 3 warm-up rows)
 
 struct SweepArgs {
     DiaMat A;                      // fine level: 7 fp32 planes + the fp32 Jacobi scaling plane
@@ -56,7 +62,7 @@ __device__ __forceinline__ void sw_gather(const T (*ring)[kSwThreads], int u, in
     xv[5] = up[tx]; xv[6] = up[tx + 1];
 }
 
-__global__ void __launch_bounds__(kSwThreads, 4)
+__global__ void __launch_bounds__(kSwThreads, 8)
     k_mg_down(SweepArgs S, const double *__restrict__ b, double *__restrict__ xpre, double *__restrict__ rc) {
     __shared__ double sq[4][kSwThreads];     // dinv_j b_j (PRE2's scaled right-hand side)
     __shared__ double sx[4][kSwThreads];     // x_pre
@@ -160,7 +166,7 @@ __global__ void __launch_bounds__(kSwThreads, 4)
     }
 }
 
-__global__ void __launch_bounds__(kSwThreads, 3)
+__global__ void __launch_bounds__(kSwThreads, 6)
     k_mg_up(SweepArgs S, const double *__restrict__ b, const double *__restrict__ xpre, const double *__restrict__ xc,
             double *__restrict__ x) {
     __shared__ double sx1[8][kSwThreads];    // x1 = x_pre + P xc
@@ -268,7 +274,8 @@ static bool mgsweep_ok(const femo_problem *L, const femo_problem *C, const MgPar
            L->state.ndofs > g_env.mgfused_max_rows;
 }
 
-// strips of near-equal even width, and bands of coarse rows sized so that the grid is about one wave of resident CTAs;
+// strips of near-equal even width, and bands of coarse rows sized so that the grid is about one wave of resident CTAs
+// (small levels: bands of one coarse row, more than a wave of short CTAs);
 // the degree-2 Chebyshev coefficients (both sweeps use c0, c1, c2)
 static int mgsweep_args(const femo_problem *L, const femo_problem *C, const void *kern, const MgParams &mp, SweepArgs &S,
                         dim3 &grid) {
